@@ -5,6 +5,7 @@
   python bench.py --impl reference --gpus N --steps K ...  CPU arm: the oracle port of the reference loop on host cores
   python bench.py --config lq|evaporation|unicycle|awe9 ...  the other BASELINE.json configs at their own batch sizes
   python bench.py --scaling strong ...                     fixed 2^20 instances in total, split over the ranks
+  python bench.py --dump-outputs DIR ...                   also write the last timed step's u0 / status as DIR/*.npy
 
 A "step" = one pass of the hot path over one batch: `ctrl.reset(); ctrl.step(X0)` for B = 2^20 seeded initial states
 per GPU (the alpha-sweep loop of tunempc/closed_loop_tools.py:43-68 as one batched call).  Weak scaling: every rank
@@ -138,13 +139,13 @@ def _oracle_worker(args):
 def _twin_worker(args):
     """compiled CPU baseline (BASELINE.md B2): the solver source of the CUDA library compiled as a sequential host program
     (tests/twin, test infrastructure), one process per core, each on its own chunk of the sample"""
-    lo, hi, seed, name = args
+    lo, hi, seed, name, build_dir = args
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     from twin.twin import Twin
     from tunempc_b200.problem import build_tables
     pb = load_problem(name)
     X0 = sample_x0(pb, hi, seed, name)[lo:hi]
-    tw = Twin(pb, build_tables(pb))
+    tw = Twin(pb, build_tables(pb), build_dir=build_dir)
     tw.reset(hi - lo)
     t = time.perf_counter()
     o = tw.step(X0)
@@ -153,16 +154,18 @@ def _twin_worker(args):
 
 def compiled_cpu_baseline(name, per_core=48, seed=1000):
     import multiprocessing as mp
+    import tempfile
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     from twin.twin import build as twin_build
-    twin_build(name)                                       # g++ once, before the pool forks
     cores = len(os.sched_getaffinity(0))
     n = cores * per_core
-    jobs = [(c * per_core, (c + 1) * per_core, seed, name) for c in range(cores)]
-    t0 = time.perf_counter()
-    with mp.get_context("fork").Pool(cores) as pool:
-        res = pool.map(_twin_worker, jobs)
-    dt = time.perf_counter() - t0
+    with tempfile.TemporaryDirectory(prefix="tmpc_twin_") as d:   # the benchmark writes nothing into the tree (it may be read-only)
+        jobs = [(c * per_core, (c + 1) * per_core, seed, name, d) for c in range(cores)]
+        twin_build(name, d)                                # g++ once, before the pool forks
+        t0 = time.perf_counter()
+        with mp.get_context("fork").Pool(cores) as pool:
+            res = pool.map(_twin_worker, jobs)
+        dt = time.perf_counter() - t0
     return {"value": n / dt, "unit": UNIT, "cores": cores, "kind": "port",
             "sample": "%d x0 of the same distribution (%d per core, %d converged), the CUDA library's solver source compiled with g++ -O2 "
                       "as a sequential host program (tests/twin), one process per core" % (n, per_core, sum(r[2] for r in res))}
@@ -218,6 +221,26 @@ def ncu_traffic():
         return {}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each (B, ...) array as out_dir/<name>.npy (float64) for output-by-output comparison of two builds.  Inputs are
+    seeded, so the same arguments give the same rows; above 64 MB in all, the same fixed seeded sample of rows is kept
+    from every array (its indices go to rows.npy)."""
+    host = {k: np.asarray(v.cpu().numpy() if hasattr(v, "cpu") else v, dtype=np.float64) for k, v in arrays.items()}
+    B = next(iter(host.values())).shape[0]
+    row_bytes = sum(a[0].nbytes for a in host.values())
+    if B * row_bytes > DUMP_LIMIT_BYTES:
+        n = (DUMP_LIMIT_BYTES - 4096) // (row_bytes + 8)            # 4 KB for the .npy headers
+        rows = np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+        host = {k: a[rows] for k, a in host.items()}
+        host["rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -230,7 +253,14 @@ def main():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"], help="strong: the batch is the TOTAL, split over the ranks")
     ap.add_argument("--hessian", default="exact")
     ap.add_argument("--cpu-sample", type=int, default=40, help="x0 of the batch timed on the CPU oracle port (about 12 s)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (u0, status) as DIR/<name>.npy, to compare two builds "
+                         "(B200 arm on one GPU only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs writes the outputs of the B200 arm on one GPU: not with --impl reference or more than one rank")
     if args.impl == "reference":
         run_reference_arm(args)
         return
@@ -309,11 +339,13 @@ def main():
     e1 = torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(K):
-        one_step(X0_dev[i % nbatches], count=True)
+        U_last = one_step(X0_dev[i % nbatches], count=True)
     e1.record()
     barrier()
     ms_dev = e0.elapsed_time(e1)
     status = ctrl.status
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"u0": U_last, "status": status})
     flags = ctrl.log["flags"][-1]
     stat_hist = torch.bincount(status.to(torch.int64), minlength=6)[:6].to(torch.float64)
     # per-bit counts: [no flag, GN fallback (1), damped step (2), GN re-solve (4), non-convex primal step (8)]

@@ -68,12 +68,23 @@ class StageLib:
 _qpo = None
 
 
+class NonConvexQP(np.linalg.LinAlgError):
+    """the dense solver's QP is not convex where it would have to be (see qp_dense)"""
+
+
+class _NotPositiveDefinite(np.linalg.LinAlgError):
+    """the reduced Hessian of the Goldfarb-Idnani solve has no Cholesky factor"""
+
+
 def qpoases_available():
     return os.path.exists(os.path.join(_HERE, "_ref", "libqpoases_e.so"))
 
 
-def qp_qpoases(H, g, A, lba, uba):
-    """the reference tree's vendored qpOASES_e (oracle/_ref/libqpoases_e.so via oracle/qpoases_shim.c)."""
+def qp_qpoases(H, g, A, lba, uba, lam_hint=None, info=None):
+    """the reference tree's vendored qpOASES_e (oracle/_ref/libqpoases_e.so via oracle/qpoases_shim.c), cold-started as in
+    the reference: lam_hint is not used."""
+    if info is not None:
+        info["branch"] = "qpoases"
     global _qpo
     if _qpo is None:
         _qpo = ctypes.CDLL(os.path.join(_HERE, "_ref", "libqpoases_e.so"))
@@ -95,10 +106,86 @@ def qp_qpoases(H, g, A, lba, uba):
     return x, lam
 
 
-def qp_dense(H, g, A, lba, uba, tol=1e-11):
+def qp_dense(H, g, A, lba, uba, lam_hint=None, info=None, tol=1e-11):
     """own dense solver: null-space elimination of the equality rows, then Goldfarb-Idnani dual active set on the
-    reduced strictly convex problem.  Exact (active-set) solution: inactive multipliers are exact zeros."""
+    reduced strictly convex problem.  Exact (active-set) solution: inactive multipliers are exact zeros.
+
+    A reduced Hessian that is not positive definite is first made so, only to find the active set; the QP is then
+    re-solved on that active set with the original H (exact, free of the modification) and the result is accepted only
+    as a KKT point of the original QP:
+      - positive semidefinite (slack columns without curvature): a small proximal term on the null space;
+      - indefinite (exact Hessian after the 'reduced' regularisation, which makes it positive definite only with the rows
+        active in lam_hint held as well): rho/2 |A_S d - b_S|^2 over those held rows S, which vanishes with its gradient
+        wherever they sit on their bounds, so the local minimiser on which they stay there is the one found.
+    The point returned satisfies the second-order condition too: the reduced Hessian on its active set is positive
+    semidefinite (a saddle point is rejected).  Raises NonConvexQP when neither gives such a point.  info (a dict), when
+    given, receives the branch taken: 'gi', 'psd' or 'held'."""
     g = np.asarray(g, dtype=np.float64).ravel()
+    if info is not None:
+        info["branch"] = "gi"
+    try:
+        return _qp_dense_gi(H, g, A, lba, uba, tol)
+    except _NotPositiveDefinite:
+        pass
+    n = H.shape[0]
+    free = uba - lba != 0
+    Z = null_space(A[~free]) if (~free).any() else np.eye(n)
+    ev = np.linalg.eigvalsh(0.5 * (Z.T @ H @ Z + (Z.T @ H @ Z).T))
+    big = max(1.0, np.abs(ev).max())
+    S = None
+    if ev.min() > -1e-10 * big:
+        branch = "psd"
+        Hm, gm = H + 1e-6 * big * Z @ Z.T, g
+    else:
+        branch = "held"
+        if lam_hint is None:
+            raise NonConvexQP("QP not convex on the null space of its equality rows")
+        held = np.where(free & (lam_hint < 0) & np.isfinite(lba))[0]
+        held_up = np.where(free & (lam_hint > 0) & np.isfinite(uba))[0]
+        S = np.concatenate([held, held_up]).astype(int)
+        bS = np.concatenate([lba[held], uba[held_up]])
+        if len(S) == 0:
+            raise NonConvexQP("QP not convex on the null space of its equality rows and no held rows")
+        AS = A[S]
+        rho = big / max(np.abs(AS).max() ** 2, 1e-300)
+        for _ in range(40):
+            Hm, gm = H + rho * AS.T @ AS, g - rho * AS.T @ bS
+            if np.linalg.eigvalsh(0.5 * (Z.T @ Hm @ Z + (Z.T @ Hm @ Z).T)).min() > 0:
+                break
+            rho *= 10.0
+        else:
+            raise NonConvexQP("QP not convex on the face of its held rows")
+    if info is not None:
+        info["branch"] = branch
+    try:
+        d, lam = _qp_dense_gi(Hm, gm, A, lba, uba, tol)
+    except _NotPositiveDefinite:
+        raise NonConvexQP("QP not convex after the modification")
+    if S is not None and np.abs(A[S] @ d - bS).max() > 1e-7 * max(1.0, np.abs(bS).max()):
+        raise NonConvexQP("QP not convex and its held rows leave their bounds")
+    # the active set found: equality rows and rows with a non-zero multiplier; exact solve of its KKT system with H
+    W = np.where((~free) | (lam != 0))[0]
+    bW = np.where(lam[W] > 0, uba[W], lba[W])
+    m = len(W)
+    K = np.block([[H, A[W].T], [A[W], np.zeros((m, m))]])
+    sol = np.linalg.lstsq(K, np.concatenate([-g, bW]), rcond=None)[0]
+    d = sol[:n]
+    lam = np.zeros(A.shape[0])
+    lam[W] = sol[n:]
+    r = A @ d
+    sc = max(1.0, np.abs(np.concatenate([lba[np.isfinite(lba)], uba[np.isfinite(uba)]])).max(initial=1.0))
+    at_up = bW == uba[W]                                       # CasADi sign: lower-active <= 0, upper-active >= 0
+    wrong = free[W] & np.where(at_up, lam[W] < -1e-10 * big, lam[W] > 1e-10 * big)
+    if (np.any(r < lba - 1e-8 * sc) or np.any(r > uba + 1e-8 * sc) or wrong.any()
+            or np.abs(H @ d + g + A.T @ lam).max() > 1e-8 * max(1.0, np.abs(g).max())):
+        raise NonConvexQP("the modified QP's active set gives no KKT point of the QP")
+    ZW = null_space(A[W]) if m else np.eye(n)
+    if ZW.shape[1] and np.linalg.eigvalsh(0.5 * (ZW.T @ H @ ZW + (ZW.T @ H @ ZW).T)).min() < -1e-10 * big:
+        raise NonConvexQP("the KKT point found is a saddle point of the QP")
+    return d, lam
+
+
+def _qp_dense_gi(H, g, A, lba, uba, tol):
     n = H.shape[0]
     eq = np.where(uba - lba == 0)[0]
     lo = np.where((uba - lba != 0) & np.isfinite(lba))[0]
@@ -122,7 +209,10 @@ def qp_dense(H, g, A, lba, uba, tol=1e-11):
     gr = Z.T @ (H @ dp + g)
     Gr = G @ Z
     hr = hh - G @ dp
-    L = np.linalg.cholesky(Hr)                      # raises LinAlgError if reduced Hessian not PD
+    try:
+        L = np.linalg.cholesky(Hr)
+    except np.linalg.LinAlgError:
+        raise _NotPositiveDefinite("reduced Hessian not positive definite")
     Hinv = lambda v: np.linalg.solve(L.T, np.linalg.solve(L, v))
     y = -Hinv(gr)
     act = []                                        # indices into G rows
@@ -413,12 +503,23 @@ class Sqp:
         alpha = 0.0
         k = 0
         converged = False
+        branches = {"gi": 0, "psd": 0, "held": 0, "qpoases": 0, "gn_resolve": 0}
+        info = {}
         while not converged:                                          # :149
             g0, J = nlp.g(w0, p0, order=1)                            # :152
             H = nlp.hess(w0, p0, lam, o["hessian_approximation"])     # :330
             if o["regularization"] == "reduced":
                 H = self._regularize(H, J, lam)                       # :155
-            d, lam_new = self.qp(H, nlp.jacf(w0, p0), J, nlp.lbg - g0, nlp.ubg - g0)   # :158-168
+            try:
+                d, lam_new = self.qp(H, nlp.jacf(w0, p0), J, nlp.lbg - g0, nlp.ubg - g0, lam, info)   # :158-168
+            except NonConvexQP:
+                # qpOASES follows its homotopy through a QP that is not convex; the dense solver cannot.  Like the device
+                # solver (DESIGN.md), re-solve this iteration with the Gauss-Newton Hessian (economic NLPs have none: raises
+                # again).  Converged points stay those of the reference, the iteration path may not.
+                branches["gn_resolve"] += 1
+                H = nlp.hess(w0, p0, lam, "gauss_newton")
+                d, lam_new = self.qp(H, nlp.jacf(w0, p0), J, nlp.lbg - g0, nlp.ubg - g0, lam, info)
+            branches[info["branch"]] += 1
             self.n_qp += 1
             # line search (:289-325)
             alpha = 1.0
@@ -456,7 +557,10 @@ class Sqp:
         nAC = len([i for i in as_init if i not in as_idx]) + len([i for i in as_idx if i not in as_init])
         self.stats = {"x": w0, "lam_g": lam, "iter_count": k, "f": nlp.f(w0, p0), "nAC": nAC, "nAS": len(as_idx),
                       "status": status, "alpha": alpha, "min_eig": min_eig, "filter": np.array(filt),
-                      "dual_infeas": dual, "as_idx": as_idx}
+                      "dual_infeas": dual, "as_idx": as_idx,
+                      # QP solves per branch of qp_dense (or qpOASES); gn_resolve counts iterations re-solved with the
+                      # Gauss-Newton Hessian, where the iteration path is no longer the reference's
+                      "qp_branches": branches}
         return {"x": w0, "lam_g": lam, "S": {"H": H}}
 
 

@@ -123,6 +123,66 @@ def test_qp_solvers_agree(rp):
         assert set(np.nonzero(l1[me:])[0]) == set(np.nonzero(l2[me:])[0])
 
 
+def test_qp_dense_semidefinite_known_answer(rp):
+    """min 1/2 x^2 + 2 s  s.t.  y - x = 0, x + s >= 1, s >= 0 over (x, y, s): no curvature in y and s, so the reduced Hessian
+    is only semidefinite.  Answer by hand: x = y = 1, s = 0; lam = (0, -1, -1) (lower-active => negative)."""
+    H = np.diag([1.0, 0.0, 0.0])
+    g = np.array([0.0, 0.0, 2.0])
+    A = np.array([[-1.0, 1.0, 0.0], [1.0, 0.0, 1.0], [0.0, 0.0, 1.0]])
+    lba, uba = np.array([0.0, 1.0, 0.0]), np.array([0.0, np.inf, np.inf])
+    info = {}
+    d, lam = rp.qp_dense(H, g, A, lba, uba, info=info)
+    assert info["branch"] == "psd"
+    assert np.allclose(d, [1.0, 1.0, 0.0], atol=1e-12) and np.allclose(lam, [0.0, -1.0, -1.0], atol=1e-12)
+
+
+def test_qp_dense_held_rows_known_answer(rp):
+    """min 1/2 (d1^2 - d2^2 + d3^2) + 2 d2  s.t.  d3 - d1 = 0, d2 >= 1, d1 + d2 >= -5: negative curvature in d2, so the QP is
+    not convex on the null space of its equality row and is unbounded below.  With d2 >= 1 held (its multiplier in the hint)
+    the local minimiser on that face is d = (0, 1, 0), lam = (0, -1, 0): f'(d2 = 1) = 1 > 0 keeps the row active."""
+    H = np.diag([1.0, -1.0, 1.0])
+    g = np.array([0.0, 2.0, 0.0])
+    A = np.array([[-1.0, 0.0, 1.0], [0.0, 1.0, 0.0], [1.0, 1.0, 0.0]])
+    lba, uba = np.array([0.0, 1.0, -5.0]), np.array([0.0, np.inf, np.inf])
+    with pytest.raises(rp.NonConvexQP):
+        rp.qp_dense(H, g, A, lba, uba)                                      # no held rows: no convex face to start from
+    info = {}
+    d, lam = rp.qp_dense(H, g, A, lba, uba, lam_hint=np.array([0.0, -0.5, 0.0]), info=info)
+    assert info["branch"] == "held"
+    assert np.allclose(d, [0.0, 1.0, 0.0], atol=1e-12) and np.allclose(lam, [0.0, -1.0, 0.0], atol=1e-12)
+
+
+def test_qp_dense_rejects_saddle_point(rp):
+    """min 1/2 (d1^2 - d2^2)  s.t.  d2 >= 0 with d2 >= 0 held: d = 0 is a KKT point (zero multiplier) but a saddle point --
+    d2 > 0 decreases the objective -- and is not returned."""
+    with pytest.raises(rp.NonConvexQP):
+        rp.qp_dense(np.diag([1.0, -1.0]), np.zeros(2), np.array([[0.0, 1.0]]), np.array([0.0]), np.array([np.inf]),
+                    lam_hint=np.array([-1.0]))
+
+
+@pytest.mark.parametrize("name,idx,branch", [("evaporation_sc1", (0, 5, 11), "psd"), ("awe9", (0,), "psd"),
+                                             ("cstr", (4, 5), "held")])
+def test_dense_qp_branches_vs_qpoases_golden(rp, name, idx, branch):
+    """The dense QP solver's semidefinite and held-row branches against the reference's qpOASES_e: the golden fixtures were
+    computed by this oracle with qpOASES_e as its QP solver.  Soft-constrained evaporation and awe9 (slack columns without
+    curvature) take the semidefinite branch in every QP; these CSTR instances reach QPs that are not convex on the null space of the
+    equality rows.  Converged point, multipliers and active set match; the iteration count too wherever no iteration was
+    re-solved with the Gauss-Newton Hessian."""
+    pb, gold = load_problem(name), load_golden(name)
+    oc = rp.Pmpc(pb, qp="dense")
+    for b in idx:
+        oc.reset()
+        u = oc.step(gold["X0"][b])
+        br = oc.sqp.stats["qp_branches"]
+        assert br[branch] > 0 and oc.log["status"][-1] == 0, (b, br)
+        assert np.max(np.abs(u - gold["u0_t6"][b]) / np.maximum(np.abs(gold["u0_t6"][b]), 1.0)) < 1e-7
+        assert np.max(np.abs(oc.w_sol - gold["w_t6"][b]) / np.maximum(np.abs(gold["w_t6"][b]), 1.0)) < 1e-7
+        assert np.max(np.abs(oc.lam_g - gold["lam_t6"][b]) / np.maximum(np.abs(gold["lam_t6"][b]), 1.0)) < 1e-5
+        assert set(np.nonzero(oc.lam_g)[0]) == set(np.nonzero(gold["lam_t6"][b])[0]) and oc.log["nAS"][-1] == gold["nAS_t6"][b]
+        if br["gn_resolve"] == 0:
+            assert oc.log["iter"][-1] == gold["iter_t6"][b]
+
+
 def test_cstr_reference_point_and_idempotence(rp):
     pb = load_problem("cstr")
     ctrl = rp.Pmpc(pb)

@@ -173,6 +173,7 @@ def test_periodic_ocp_with_path_constraints_and_economic_mpc():
         uo = np.array([ocs[b].step(xo[b]) for b in range(3)])
         assert (o["status"] == 0).all() and all(ocs[b].log["status"][-1] == 0 for b in range(3))
         assert np.array_equal(o["iter"], [ocs[b].log["iter"][-1] for b in range(3)])
+        assert all(ocs[b].sqp.stats["qp_branches"]["gn_resolve"] == 0 for b in range(3))   # the oracle followed the reference's path
         assert np.array_equal(o["nAS"], [ocs[b].log["nAS"][-1] for b in range(3)])
         assert np.max(np.abs(o["u0"] - uo)) < 1e-10
         x, xo = st.F(x, o["u0"]), st.F(xo, uo)
@@ -233,6 +234,7 @@ def test_tuner_with_nonlinear_path_constraints():
             continue
         n_ok += 1
         assert o["status"][b] == 0 and o["iter"][b] == oc.log["iter"][-1] and o["nAS"][b] == oc.log["nAS"][-1]
+        assert oc.sqp.stats["qp_branches"]["gn_resolve"] == 0                  # the oracle followed the reference's path
         assert np.max(np.abs(o["u0"][b] - uo)) < 1e-10 and np.max(np.abs(o["w"][b] - oc.w_sol)) < 1e-9
         for k in range(pb.N):
             assert np.array_equal(o["lam"][b][pb.g_h(k)] != 0, oc.lam_g[pb.g_h(k)] != 0), (b, k)

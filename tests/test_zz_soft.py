@@ -29,6 +29,7 @@ def test_tuner_soft_constraints_gpu(built):
         uo = oc.step(X0[b])
         assert np.max(np.abs(U[b] - uo) / np.maximum(np.abs(uo), 1.0)) < 1e-6, b
         assert ctrl.log["iter"][-1].cpu().numpy()[b] == oc.log["iter"][-1]
+        assert oc.sqp.stats["qp_branches"]["gn_resolve"] == 0            # the oracle followed the reference's path
     with pytest.raises(ValueError):
         t.create_mpc("tuned", 30, opts={"slack_flag": "some"})
 
@@ -60,6 +61,7 @@ def test_periodic_path_constraint_economic_gpu(built):
         uo = np.array([ocs[b].step(xo[b]) for b in range(3)])
         assert (ctrl.status.cpu().numpy() == 0).all()
         assert np.array_equal(ctrl.log["iter"][-1].cpu().numpy(), [ocs[b].log["iter"][-1] for b in range(3)])
+        assert all(ocs[b].sqp.stats["qp_branches"]["gn_resolve"] == 0 for b in range(3))
         assert np.max(np.abs(U.cpu().numpy() - uo)) < 1e-8, s
         X = ctrl.plant_step(X, U)
         xo = st.F(xo, uo)

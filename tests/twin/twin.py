@@ -19,8 +19,9 @@ def _i(a):
     return a.ctypes.data_as(_ip)
 
 
-def build(name):
-    out = os.path.join(_HERE, "libtwin_%s.so" % name)
+def build(name, out_dir=None):
+    """g++-compile libtwin_<name>.so into out_dir (default: next to this file)"""
+    out = os.path.join(out_dir or _HERE, "libtwin_%s.so" % name)
     srcs = [os.path.join(_HERE, "twin.cpp"), os.path.join(_ROOT, "tunempc_b200/csrc/tmpc_core.cuh"),
             os.path.join(_ROOT, "tunempc_b200/csrc/tmpc_qp.cuh"),
             os.path.join(_ROOT, "tunempc_b200/csrc/gen/model_%s.h" % name)]
@@ -33,9 +34,9 @@ def build(name):
 
 
 class Twin:
-    def __init__(self, pb, tables, maxact=32, rho_rel=1e4, reg_mode=8, nonconvex_after=10, **_ignored):
+    def __init__(self, pb, tables, maxact=32, rho_rel=1e4, reg_mode=8, nonconvex_after=10, build_dir=None, **_ignored):
         self.pb, self.tab = pb, tables
-        self.lib = ctypes.CDLL(build(pb.name))
+        self.lib = ctypes.CDLL(build(pb.name, build_dir))
         self.maxact, self.rho_rel, self.reg_mode = maxact, rho_rel, int(os.environ.get("TWIN_REG_MODE", reg_mode))
         self.nonconvex_after = nonconvex_after
         self.reset(1)
