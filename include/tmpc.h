@@ -74,8 +74,10 @@ typedef struct {
   int32_t max_working_set; /* rows the dual active set may ADD to the base rows of one QP (default 32, clipped to N*nh); the base rows
                               (terminal rows + rows active in the multipliers) live in the factorisation and do not count.
                               Overflow is reported per instance as status TMPC_WS_OVERFLOW, never as "infeasible" */
-  int32_t economic;        /* 1: economic MPC -- stage cost = the compiled model's l(x,u), exact Hessian forced (pmpc.py:97-107,
-                              173-183, 299-301); 0: tuned / tracking cost from the H, q tables (mtools.py:43-57) */
+  int32_t economic;        /* 1: economic MPC -- stage cost = the compiled model's l(x,u) + scost'usc, exact Hessian forced
+                              (pmpc.py:97-107, 173-183, 299-301, 338-339): H and the (x,u,us) entries of q are ignored (pass
+                              zeros), the usc entries of q still carry scost; 0: tuned / tracking cost from the H, q tables
+                              (mtools.py:43-57) */
 } tmpc_opts;
 
 void tmpc_default_opts(tmpc_opts* o);

@@ -230,9 +230,14 @@ def awe9():
                 gnl_x_idx=[0], w_guess=card["w_guess"])
 
 
-def awe9_problem(stage_F, N=None, hessian_approximation="exact"):
+def awe9_problem(stage_F, N=None, hessian_approximation="exact", mpc_type="tuned"):
     """Reference trajectory, tuning and multipliers of the awe9 stand-in (see `awe9`): simulate the forced response until it is
-    periodic, then pick multipliers on the active rows and the gradient q that makes the reference a KKT point."""
+    periodic, then pick multipliers on the active rows and the gradient q that makes the reference a KKT point.
+
+    mpc_type='economic' mirrors `make_problem`: stage cost = the card's l(x,u) (+ scost'usc), H = q = 0, exact Hessian, the same
+    lam_h_ref, lam_g_ref and scost, lam_dyn_ref = 0.  That is a problem of the shape of the paper's AWE economic MPC (nx 9, nu 3,
+    ns 3, nsc 3, N 20, p 40, exact Hessian of a non-tracking cost).  It is not an economic optimum: the reference stays the
+    forced periodic response, so the controller does not return u_ref at x_ref."""
     import sympy as sp
     from .problem import MpcProblem
     cfg = awe9()
@@ -291,6 +296,11 @@ def awe9_problem(stage_F, N=None, hessian_approximation="exact"):
                     lam_dyn_ref=np.zeros((P, nx)), term_idx=list(cfg["term_idx"]), S_A=np.array(Ss[:, :, :nx]),
                     S_B=np.array(Ss[:, :, nx:]), hessian_approximation=hessian_approximation, mpc_type="tuned",
                     ns=ns, nsc=nsc, scost=scost, lam_g_ref=lam_g, gnl_x_idx=list(cfg["gnl_x_idx"]))
+    if mpc_type == "economic":
+        pb.mpc_type = "economic"
+        pb.hessian_approximation = "exact"
+        pb.H = np.zeros_like(pb.H)
+        pb.q = np.zeros_like(pb.q)
     info = {"cfg": cfg, "periodicity_error": float(np.max(np.abs(x - X[0]))), "active": act, "hval": hval}
     return pb, info
 
@@ -363,7 +373,7 @@ def make_problem(name, stage_F, N=None, hessian_approximation="exact", mpc_type=
     from .problem import MpcProblem
 
     if name == "awe9":
-        return awe9_problem(stage_F, N=N, hessian_approximation=hessian_approximation)
+        return awe9_problem(stage_F, N=N, hessian_approximation=hessian_approximation, mpc_type=mpc_type)
     cfg = CONFIGS[name]()
     model = cfg["model"]
     nx, nu = model.nx, model.nu

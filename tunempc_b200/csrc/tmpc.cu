@@ -454,11 +454,6 @@ int tmpc_create(tmpc_handle** out, const tmpc_dims* dims, const tmpc_opts* opts,
     delete h;
     return 2;
   }
-  if (opts && opts->economic && (NS > 0 || NSC > 0)) {
-    fprintf(stderr, "tmpc_create: the economic stage cost is defined on (x,u) only: no slack variables\n");
-    delete h;
-    return 2;
-  }
   int ndev = 0;
   cudaError_t e = cudaGetDeviceCount(&ndev);
   if (e != cudaSuccess || device >= ndev) {

@@ -841,6 +841,8 @@ TM_HD void tm_eval_point(const TmProb& P, const TmState& S, int64_t inst, double
     double fk = 0.0;
     if (P.economic) {
       fk = tmpc_stage_cost(z, z + NX);
+#pragma unroll
+      for (int b = NZM + NS; b < NZ; ++b) fk += qk[b] * z[b];    // scost'usc (pmpc.py:338-339)
     } else {
 #pragma unroll
       for (int a = 0; a < NZ; ++a) {
@@ -920,7 +922,9 @@ TM_HD double tm_dual_infeas(const TmProb& P, const TmState& S, int64_t inst) {
       double z[NZ];
 #pragma unroll
       for (int b = 0; b < NZ; ++b) { z[b] = w[k * NZ + b]; gl[b] = 0.0; }
-      tmpc_cost_grad(z, z + NX, gl);
+      tmpc_cost_grad(z, z + NX, gl);                              // dl/d(x,u); 0 on us
+#pragma unroll
+      for (int b = NZM + NS; b < NZ; ++b) gl[b] = qk[b];          // scost on usc
     }
 #if NS > 0
     double Jg[NS * NZM];

@@ -1636,20 +1636,26 @@ TM_HD void tm_qp_setup(const TmProb& P, const TmState& S, int64_t inst, TmQpWs& 
   }
   for (int e = lane; e < N * NX; e += TM_NL) { int k = e / NX, a = e % NX; s.b[e] = lin[(size_t)k * TM_LSZ + a] - w[(k + 1) * NZ + a]; }
   if (P.economic) {
-    // economic stage cost: Q_k = d2l/dz2 (+ lam' d2F), r_k = dl/dz at the iterate
+    // economic stage cost l(x,u) + scost'usc (pmpc.py:299-301,338-339): Q_k = d2l/d(x,u)2 (+ lam' d2F) on the (x,u) block and
+    // zero on the slacks, r_k = (dl/d(x,u), 0_ns, scost) at the iterate.  l lives on (x,u) only: tmpc_cost_grad / _hess write
+    // NZM / NZM x NZM values.  scost comes from the usc entries of q (MpcProblem.device_tables).
     for (int k = lane; k < N; k += TM_NL) {
-      double z[NZ], gl[NZ], Hl[NZ * NZ];
+      const double* qk = P.q + (size_t)((S.phase + k) % P.p) * NZ;
+      double z[NZ], gl[NZM], Hl[NZM * NZM];
 #pragma unroll
       for (int b = 0; b < NZ; ++b) z[b] = w[k * NZ + b];
       tmpc_cost_grad(z, z + NX, gl);
       tmpc_cost_hess(z, z + NX, Hl);
       for (int i = 0; i < NZ; ++i) {
         for (int j = 0; j < NZ; ++j) {
-          double v = 0.5 * (Hl[i * NZ + j] + Hl[j * NZ + i]);
-          if (use_exact) v += lin[(size_t)k * TM_LSZ + NX + NX * NZM + (i <= j ? tm_pair_idx(i, j) : tm_pair_idx(j, i))];
+          double v = 0.0;
+          if (i < NZM && j < NZM) {
+            v = 0.5 * (Hl[i * NZM + j] + Hl[j * NZM + i]);
+            if (use_exact) v += lin[(size_t)k * TM_LSZ + NX + NX * NZM + (i <= j ? tm_pair_idx(i, j) : tm_pair_idx(j, i))];
+          }
           s.Q[(size_t)k * NZ * NZ + i * NZ + j] = v;
         }
-        s.r[k * NZ + i] = gl[i];
+        s.r[k * NZ + i] = i < NZM ? gl[i] : (i < NZM + NS ? 0.0 : qk[i]);
       }
     }
   } else {

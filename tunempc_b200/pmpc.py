@@ -69,10 +69,10 @@ def problem_from_reference_args(N, sys, cost, wref, tuning, lam_g_ref, sensitivi
     else:
         w = np.atleast_2d(np.asarray(wref, dtype=np.float64))
     P = w.shape[0]
-    if economic and (ns or nsc):
-        raise NotImplementedError("economic MPC with slack variables is not built (the device evaluates l on (x,u) only)")
     if economic:
-        H, q = np.zeros((P, nzr, nzr)), np.zeros((P, nzr))                                     # pmpc.py:103: no tuning required
+        # pmpc.py:103: no tuning required.  With slacks the stage cost is l(x,u) + scost'usc (pmpc.py:299-301,338-339): H and
+        # q stay zero on (x,u,us) and device_tables() puts scost into the usc entries of q
+        H, q = np.zeros((P, nzr, nzr)), np.zeros((P, nzr))
     else:
         assert tuning is not None, "Provide tuning matrices for tracking MPC!"                # pmpc.py:118
         Hs = [np.asarray(h, dtype=np.float64) for h in tuning["H"]]
