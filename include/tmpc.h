@@ -124,6 +124,26 @@ int tmpc_busy(tmpc_handle* h, int32_t* busy);
 int tmpc_step_host(tmpc_handle* h, const double* X0_host, int64_t B, double* U0_host, double* W_host,
                    double* LAM_host, double* G_host, int32_t* status_host, int32_t* iter_host, int32_t* flags_host);
 
+/* Feedback Jacobian J_b = du0*_b / dx0_b of the solutions of the last tmpc_step / tmpc_step_host / (tmpc_step_async + tmpc_wait),
+ * the quantity the tuned controller is built to match (first-order equivalence with the economic controller).
+ * Definition: at instance b's solution (w*, lam*) the held set A is every equality row (init, dynamics, nonlinear rows g, terminal
+ * rows) plus every inequality row with lam* != 0, except the rows relax0 drops at stage 0.  J_b is the u_0 block of dw in
+ *     [H  J_A'; J_A  0] [dw; dlam] = [0; e_j on the init rows],   j = 0 .. nx-1,
+ * with H the exact Hessian of the Lagrangian and J_A the Jacobian of the held rows: the derivative of the solution map (implicit
+ * function theorem) under strict complementarity, the active set held.
+ * Layout: J[b*nu*nx + i*nx + j] = d u0_i / d x0_j (B x nu x nx, row-major); jstatus (B) per instance, values below.
+ * Buffers: host memory if dst_is_host != 0, else device memory on the handle's device (runs on `cuda_stream`).  Returns after
+ * its kernels have finished.  Leaves the warm start, the phase index, the log, counters and timing unchanged.
+ * API errors: no step has finished since tmpc_create / tmpc_reset; a step is in flight; the handle uses the Gauss-Newton
+ * Hessian (hessian_exact = 0 and not economic).  After a step with B = 0 it returns 0 and writes nothing.
+ * Cost: about nx QP solves per instance (one factorisation per column). */
+#define TMPC_JAC_OK 0          /* computed, strict complementarity holds                                                    */
+#define TMPC_JAC_WEAK 1        /* computed, but a held row has |lam| < opts.lam_tresh or a row neither held nor relaxed has
+                                  h(w*) < 10*opts.tol: the solution map has a kink there; J holds the active set as defined  */
+#define TMPC_JAC_NOT_SOLVED 2  /* the step's status is not TMPC_OK: J is NaN                                                */
+#define TMPC_JAC_SINGULAR 3    /* held rows dependent or reduced Hessian not positive definite: J is NaN                     */
+int tmpc_feedback_jacobian(tmpc_handle* h, double* J, int32_t* jstatus, int dst_is_host, void* cuda_stream);
+
 /* plant = model integrator: Xn_dev[b] = F(X_dev[b], U_dev[b])   (closed_loop_tools.py:102) */
 int tmpc_plant_step(tmpc_handle* h, const double* X_dev, const double* U_dev, int64_t B, double* Xn_dev,
                     void* cuda_stream);

@@ -34,9 +34,11 @@
 #define NU TMPC_NUM
 #include "tmpc_lin2.cuh"
 
-// thread-per-instance QP kernel (tmpc_qp_thread.cu)
+// thread-per-instance QP kernel (tmpc_qp_thread.cu) and feedback Jacobian (tmpc_fbjac_thread.cu)
 cudaError_t tm_launch_qp_thread(const TmProb& P, const TmState& S, const int* list, int cnt, const int* cnt_dev,
                                 double* wsbase, size_t ws_per_inst, int nblocks, int* work_counter, cudaStream_t st);
+cudaError_t tm_launch_fbjac_thread(const TmProb& P, const TmState& S, int cnt, double* wsbase, size_t ws_per_inst, int nblocks,
+                                   int* work_counter, double* J, int* jst, cudaStream_t st);
 int tm_qp_thread_block();
 
 #define QP_WARPS 2          /* warps (instances) per CTA in the warp-per-instance kernels */
@@ -91,6 +93,12 @@ struct tmpc_handle {
   void* host_pinned = nullptr;      // 4 + TM_NCNT words: per-iteration counts and the counters of the step
   cudaStream_t istream = nullptr;
   cudaEvent_t ev_in = nullptr;
+  // ---- feedback Jacobian (tmpc_feedback_jacobian)
+  bool solved = false;              // a step has finished since tmpc_create / tmpc_reset: its solutions are in Wsh / Lsh, LIN
+  bool fbjac_smem = false;          // k_fbjac's dynamic shared-memory limit raised
+  double* jac_buf = nullptr;        // device staging of J and jstatus for host destinations
+  int* jst_buf = nullptr;
+  int64_t jac_cap = 0;
 };
 
 static int fail(tmpc_handle* h, const char* what, cudaError_t e) {
@@ -180,6 +188,20 @@ __global__ void __launch_bounds__(QP_WARPS * 32) k_qp(TmProb P, TmState S, const
   for (int64_t slot = (int64_t)blockIdx.x * W + wid; slot < cnt; slot += (int64_t)gridDim.x * W) {   // 1 or QP_WARPS instances per CTA
     const int64_t inst = list ? list[slot] : slot;
     tm_qp(P, S, inst, ws);
+    __syncwarp();
+  }
+}
+
+// feedback Jacobian du0/dx0 at the solutions of the last step (tm_feedback_jacobian): warp per instance on the k_qp workspace
+__global__ void __launch_bounds__(QP_WARPS * 32) k_fbjac(TmProb P, TmState S, int cnt, double* cold, double* J, int* jst) {
+  extern __shared__ double smem[];
+  const int wid = threadIdx.x / 32, W = blockDim.x / 32;
+  const size_t cper = tm_qpws_cold_doubles(P.N, P.nh, P.nxt, P.maxact);
+  const size_t per = tm_qpws_doubles(P.N, P.nh, P.nxt, P.maxact) - cper;
+  TmQpWs ws;
+  tm_qpws_carve(smem + (size_t)wid * per, P.N, P.nh, P.nxt, P.maxact, ws, cold + ((size_t)blockIdx.x * W + wid) * cper);
+  for (int64_t inst = (int64_t)blockIdx.x * W + wid; inst < cnt; inst += (int64_t)gridDim.x * W) {
+    tm_feedback_jacobian(P, S, inst, ws, J, jst);
     __syncwarp();
   }
 }
@@ -619,6 +641,8 @@ void tmpc_destroy(tmpc_handle* h) {
   if (h->q0.MCOL) cudaFree(h->q0.MCOL);
   if (h->q0.bad) cudaFree(h->q0.bad);
   if (h->P.prof_counters) cudaFree(h->P.prof_counters);
+  if (h->jac_buf) cudaFree(h->jac_buf);
+  if (h->jst_buf) cudaFree(h->jst_buf);
   if (h->ev_ok) for (int i = 0; i < 8; ++i) cudaEventDestroy(h->ev[i]);
   delete h;
 }
@@ -718,6 +742,7 @@ int tmpc_reset(tmpc_handle* h, int64_t B) {
   if (!h->tables_set) { h->err = "tmpc_reset: tables not set"; return 1; }
   if (B < 0) { h->err = "tmpc_reset: negative batch size"; return 1; }
   cudaSetDevice(h->device);
+  h->solved = false;
   if (B == 0) { h->index = 0; h->S.B = 0; h->uniform_ws = true; return 0; }
   if (ensure_capacity(h, B)) return 1;
   h->index = 0;
@@ -753,8 +778,9 @@ int tmpc_step(tmpc_handle* h, const double* X0_dev, int64_t B, double* U0_dev, d
   if (!h) return 1;
   if (B < 0) { h->err = "tmpc_step: negative batch size"; return 1; }
   if (!h->tables_set || h->cap < B || h->S.B != B) { h->err = "tmpc_step: call tmpc_reset(B) first"; return 1; }
-  if (B == 0) { h->index += 1; return 0; }                   // empty batch: nothing to solve, the phase still advances
+  if (B == 0) { h->index += 1; h->solved = true; return 0; }   // empty batch: nothing to solve, the phase still advances
   cudaSetDevice(h->device);
+  h->solved = false;                                         // set again once this step has finished
   cudaStream_t st = (cudaStream_t)cuda_stream;
   TmProb& P = h->P;
   TmState& S = h->S;
@@ -902,6 +928,7 @@ int tmpc_step(tmpc_handle* h, const double* X0_dev, int64_t B, double* U0_dev, d
   CK(cudaStreamSynchronize(st));
   { double* t = S.W; S.W = h->Wsh; h->Wsh = t; }
   { double* t = S.LAM; S.LAM = h->Lsh; h->Lsh = t; }
+  h->solved = true;
   h->index += 1;                                             // pmpc.py:415
   CK(cudaEventElapsedTime(&ms, h->ev[6], h->ev[7]));
   h->timing_ms[0] = ms_lin; h->timing_ms[1] = ms_qp; h->timing_ms[2] = ms_post; h->timing_ms[3] = ms;
@@ -1012,6 +1039,57 @@ int tmpc_step_host(tmpc_handle* h, const double* X0_host, int64_t B, double* U0_
   if (status_host) CK(cudaMemcpy(status_host, h->S.status, b * sizeof(int), cudaMemcpyDeviceToHost));
   if (iter_host) CK(cudaMemcpy(iter_host, h->S.iter, b * sizeof(int), cudaMemcpyDeviceToHost));
   if (flags_host) CK(cudaMemcpy(flags_host, h->S.flags, b * sizeof(int), cudaMemcpyDeviceToHost));
+  return 0;
+}
+
+int tmpc_feedback_jacobian(tmpc_handle* h, double* J, int32_t* jstatus, int dst_is_host, void* cuda_stream) {
+  if (!h) return 1;
+  if (step_in_flight(h)) { h->err = "tmpc_feedback_jacobian: a step started by tmpc_step_async is still in flight (call tmpc_wait first)"; return 1; }
+  if (!h->P.hessian_exact) { h->err = "tmpc_feedback_jacobian: needs the exact Hessian (a Gauss-Newton controller's linearisation has no second-order term)"; return 1; }
+  if (!h->solved) { h->err = "tmpc_feedback_jacobian: no step has finished since tmpc_create / tmpc_reset"; return 1; }
+  const int64_t B = h->S.B;
+  if (B == 0) return 0;
+  if (!J || !jstatus) { h->err = "tmpc_feedback_jacobian: J and jstatus are required"; return 1; }
+  cudaSetDevice(h->device);
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  const TmProb& P = h->P;
+  double* Jd = J;
+  int* jsd = (int*)jstatus;
+  if (dst_is_host) {
+    if (h->jac_cap < B) {
+      if (h->jac_buf) cudaFree(h->jac_buf);
+      if (h->jst_buf) cudaFree(h->jst_buf);
+      h->jac_buf = nullptr; h->jst_buf = nullptr; h->jac_cap = 0;
+      CK(cudaMalloc(&h->jac_buf, (size_t)B * NUM * NX * sizeof(double)));
+      CK(cudaMalloc(&h->jst_buf, (size_t)B * sizeof(int)));
+      h->jac_cap = B;
+    }
+    Jd = h->jac_buf;
+    jsd = h->jst_buf;
+  }
+  // the solutions of the last step: after its warm-start shift they live in Wsh / Lsh; LIN still holds the linearisation at
+  // them (nothing after a step's convergence test writes LIN, D or LAMQ before the next step).  X0 only has to be a valid
+  // buffer (the perturbed solves replace the x_0 offset): the staging buffer, never the caller's pointer of the last step.
+  TmState Sc = h->S;
+  Sc.W = h->Wsh;
+  Sc.LAM = h->Lsh;
+  Sc.X0 = h->X0buf;
+  const bool use_thread = h->qp_mode == 1 || (h->qp_mode == 2 && B >= h->qp_thread_min);
+  if (use_thread) {
+    CK(tm_launch_fbjac_thread(P, Sc, (int)B, h->qp_ws, h->qp_ws_per_inst, h->qp_blocks, h->qp_counter, Jd, jsd, st));
+  } else {
+    if (!h->fbjac_smem) {
+      CK(cudaFuncSetAttribute(k_fbjac, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->qp_smem));
+      h->fbjac_smem = true;
+    }
+    k_fbjac<<<(unsigned)std::min<int64_t>((B + h->qp_warps - 1) / h->qp_warps, h->qp_wgrid), h->qp_warps * 32, h->qp_smem, st>>>(P, Sc, (int)B, h->qp_cold, Jd, jsd);
+    CK(cudaGetLastError());
+  }
+  if (dst_is_host) {
+    CK(cudaMemcpyAsync(J, Jd, (size_t)B * NUM * NX * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(jstatus, jsd, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost, st));
+  }
+  CK(cudaStreamSynchronize(st));
   return 0;
 }
 

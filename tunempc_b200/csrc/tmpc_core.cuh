@@ -1375,6 +1375,69 @@ TM_HD void tm_pd_check(const TmProb& P, const TmState& S, int64_t inst, TmQpWs& 
   TM_SYNC();
 }
 
+// Feedback Jacobian du0*/dx0 of a converged instance (tmpc_feedback_jacobian, include/tmpc.h).  Held set A = the equality rows +
+// the inequality rows with a non-zero multiplier (stage-0 rows of relax0 excluded), as in tm_pd_check.  Column j is the u_0 block
+// of the linear response of the base QP at the solution (exact Hessian, rows of A held, every offset zero) to the x_0 offset e_j:
+// the KKT system [H J_A'; J_A 0] [dw; dlam] = [0; e_j on the init rows], i.e. the implicit-function derivative of the solution
+// map under strict complementarity.  Same perturbed solve as the tabulation of the first QP (tm_qp0_build_row).  LIN must be
+// valid at (W, LAM); S.D / S.LAMQ of the instance are used as scratch.  J: B*NUM*NX, row-major (nu, nx) per instance; jst: B.
+#define TMPC_JAC_OK 0                   /* the jstatus values of include/tmpc.h (the CPU twin compiles this file without it) */
+#define TMPC_JAC_WEAK 1
+#define TMPC_JAC_NOT_SOLVED 2
+#define TMPC_JAC_SINGULAR 3
+TM_HD void tm_feedback_jacobian(const TmProb& P, const TmState& S, int64_t inst, TmQpWs& ws, double* J, int* jst) {
+  const int lane = TM_LANE;
+  const int NI = P.N * P.nh;
+  double* Ji = J + inst * (int64_t)(NUM * NX);
+  int res = TMPC_JAC_NOT_SOLVED;
+  if (S.status[inst] == 0) {
+    unsigned mask[TM_ALW];
+    for (int wd = 0; wd < TM_ALW; ++wd) mask[wd] = 0u;
+    const double* lam = S.LAM + inst * P.n_g;
+    for (int e = 0; e < NI; ++e) {
+      const int k = e / P.nh, i = e % P.nh;
+      if (k == 0 && P.relax0[i]) continue;
+      if (lam[tm_gh(P, k) + i] != 0.0) tm_mask_set(mask, e);
+    }
+    tm_pin_soft_slacks(P, mask);
+    tm_qp_setup(P, S, inst, ws, 1);
+    // strict complementarity: every held row with a multiplier above lam_tresh, every other row strictly inactive
+    int weak = 0;
+    for (int e = lane; e < NI; e += TM_NL) {
+      const int k = e / P.nh, i = e % P.nh;
+      if (k == 0 && P.relax0[i]) continue;
+      if (tm_mask_get(mask, e)) weak |= fabs(lam[tm_gh(P, k) + i]) < P.lam_tresh;
+      else weak |= ws.hv[e] < 10.0 * P.tol;
+    }
+    weak = tm_wany(weak);
+    // the perturbed solve zeroes the gradient, the dynamics defects and the terminal residuals; the residuals of the held rows
+    // and of the nonlinear rows are O(tol) at a solution and would enter every column
+    TM_SYNC();
+    for (int e = lane; e < NI; e += TM_NL) ws.hv[e] = 0.0;
+#if NS > 0
+    for (int e = lane; e < P.N * NS; e += TM_NL) ws.gv[e] = 0.0;
+#endif
+    TM_SYNC();
+    TmQpPert pt;
+    pt.homog = 1;
+    pt.row = -1;
+    pt.dout = S.D + inst * P.n_w;
+    pt.lout = S.LAMQ + inst * P.n_g;
+    unsigned nxtm[TM_ALW];
+    res = weak ? TMPC_JAC_WEAK : TMPC_JAC_OK;
+    for (int j = 0; j < NX; ++j) {
+      pt.e0_unit = j;
+      int nwrong = 0, ngi = 0;
+      if (tm_qp_solve(P, S, inst, ws, mask, nxtm, nwrong, ngi, &pt) != 0) { res = TMPC_JAC_SINGULAR; break; }
+      for (int i = lane; i < NUM; i += TM_NL) Ji[i * NX + j] = pt.dout[NX + i];
+    }
+  }
+  if (res >= TMPC_JAC_NOT_SOLVED)
+    for (int e = lane; e < NUM * NX; e += TM_NL) Ji[e] = NAN;
+  if (lane == 0) jst[inst] = res;
+  TM_SYNC();
+}
+
 // The QP of one SQP iteration for one instance.  Base rows = the inequality rows active in the current multipliers
 // (the reference's reduced space, sqp_method.py:338-341,417-423).  Outcomes of the base factorisation:
 //   positive definite                      -> solve; base rows that come back with a wrong-signed multiplier are released

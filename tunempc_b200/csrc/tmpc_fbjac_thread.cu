@@ -1,0 +1,35 @@
+// tmpc_fbjac_thread.cu -- the feedback Jacobian (tm_feedback_jacobian) as one thread per instance, on the workspace of the
+// thread-per-instance QP kernel.  A translation unit of its own: tm_qp_solve is __noinline__, and a caller with a perturbation
+// in tmpc_qp_thread.cu would change the code of that file's copy, which k_qp_thread runs.
+#include "tmpc_qp_thread.cuh"
+
+// feedback Jacobian du0/dx0 at the solutions of the last step (tm_feedback_jacobian), thread per instance on the same workspace:
+// the same CTA size and register budget, at most `nblocks` CTAs (the workspace is sized by that grid)
+__global__ void __launch_bounds__(QT_THREADS, QT_MINB) k_fbjac_thread(TmProb P, TmState S, int cnt, double* wsbase, size_t ws_per_inst,
+                                                             int* work_counter, double* J, int* jst) {
+  const int lane = threadIdx.x & 31;
+  const size_t gwarp = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  double* base = wsbase + gwarp * ws_per_inst * 32 + lane;
+  TmQpWs ws;
+  tm_qpws_carve(base, P.N, P.nh, P.nxt, P.maxact, ws);
+  double lscr[TM_QP_LSCR];
+  tm_qpws_local(lscr, ws);
+  for (;;) {
+    int start = 0;
+    if (lane == 0) start = atomicAdd(work_counter, 32);
+    start = __shfl_sync(0xffffffffu, start, 0);
+    if (start >= cnt) break;
+    const int slot = start + lane;
+    if (slot < cnt) tm_feedback_jacobian(P, S, slot, ws, J, jst);
+    __syncwarp();
+  }
+}
+
+cudaError_t tm_launch_fbjac_thread(const TmProb& P, const TmState& S, int cnt, double* wsbase, size_t ws_per_inst, int nblocks,
+                                   int* work_counter, double* J, int* jst, cudaStream_t st) {
+  cudaError_t e = cudaMemsetAsync(work_counter, 0, sizeof(int), st);
+  if (e != cudaSuccess) return e;
+  const int need = (cnt + QT_THREADS - 1) / QT_THREADS;
+  k_fbjac_thread<<<need < nblocks ? need : nblocks, QT_THREADS, 0, st>>>(P, S, cnt, wsbase, ws_per_inst, work_counter, J, jst);
+  return cudaGetLastError();
+}

@@ -266,7 +266,7 @@ class Pmpc:
         fl = np.empty(B, dtype=np.int32)
         vp = lambda t: ctypes.c_void_p(t.ctypes.data) if t is not None else None
         self.__check(L.tmpc_step_host(self.__h, vp(X0), B, vp(U0), vp(W), vp(LAM), vp(G), vp(st), vp(it), vp(fl)))
-        self.__out = dict(u0=U0, w=W, lam_g=LAM, g=G, status=st, iter=it, flags=fl)
+        self.__out = dict(u0=U0, w=W, lam_g=LAM, g=G, status=st, iter=it, flags=fl, single=single_shape is not None)
         self.__log_append()
         self.__index += 1
         if single_shape is not None:
@@ -356,6 +356,35 @@ class Pmpc:
         outs = [np.empty(B, dtype=dt) for dt in (np.float64, np.int32, np.int32, np.int32)]
         self.__check(L.tmpc_get_log(self.__h, *[ctypes.c_void_p(t.ctypes.data) for t in outs], 1))
         return outs
+
+    def feedback_jacobian(self):
+        """Feedback Jacobian du0/dx0 of the solutions of the last step (C ABI: tmpc_feedback_jacobian, definition in
+        include/tmpc.h): (J, jstatus) with J (B, nu, nx), J[b, i, j] = d u0_i / d x0_j, and jstatus (B,) int32 -- 0 ok, 1 a weakly
+        active row (the solution map has a kink; J holds the active set), 2 the step did not converge, 3 singular (J is NaN for
+        2 and 3).  torch CUDA tensors after a torch step, numpy arrays after a numpy step, ((nu, nx), int) after a single-state
+        step.  Needs the exact Hessian; leaves the warm start, the phase index and the log unchanged."""
+        if getattr(self, "_Pmpc__pending", None) is not None:
+            raise RuntimeError("feedback_jacobian: a step started by step_async is still in flight (call wait() first)")
+        pb = self.__pb
+        L = self.__lib.lib
+        B = self.__B
+        o = self.__out
+        if o is not None and type(o["u0"]).__module__.startswith("torch"):
+            import torch
+            dev = o["u0"].device
+            J = torch.empty((B, pb.nu, pb.nx), dtype=torch.float64, device=dev)
+            js = torch.empty(B, dtype=torch.int32, device=dev)
+            stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+            self.__check(L.tmpc_feedback_jacobian(self.__h, ctypes.c_void_p(J.data_ptr()), ctypes.c_void_p(js.data_ptr()), 0,
+                                                  stream))
+            return J, js
+        J = np.empty((B, pb.nu, pb.nx))
+        js = np.empty(B, dtype=np.int32)
+        self.__check(L.tmpc_feedback_jacobian(self.__h, ctypes.c_void_p(J.ctypes.data), ctypes.c_void_p(js.ctypes.data), 1,
+                                              None))
+        if o is not None and o.get("single"):
+            return J[0].copy(), int(js[0])
+        return J, js
 
     # ---- closed loop helpers -------------------------------------------------------------------------
     def plant_step(self, X, U):
