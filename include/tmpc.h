@@ -11,6 +11,7 @@
  *   tmpc_reset                      Pmpc.reset / __set_initial_guess                          (tunempc/pmpc.py:858-865, 930-948)
  *   tmpc_step / tmpc_step_host      Pmpc.step -> Sqp.solve for B initial states at once       (tunempc/pmpc.py:371-423, tunempc/sqp_method.py:136-183)
  *   tmpc_plant_step                 F(x0=x, p=u)['xf'] in closed_loop_sim                     (tunempc/closed_loop_tools.py:102)
+ *   tmpc_plant_jacobian             the first-order sensitivities of that integrator, for backpropagation through a closed loop
  *   tmpc_stage_log                  cost(x,u), h(x,u) logged per closed-loop sample            (tunempc/closed_loop_tools.py:64-65, 98-99)
  *   tmpc_get_*                      Pmpc.w_sol / g_sol / log / index properties               (tunempc/pmpc.py:1120-1142, 785-831)
  *
@@ -144,9 +145,31 @@ int tmpc_step_host(tmpc_handle* h, const double* X0_host, int64_t B, double* U0_
 #define TMPC_JAC_SINGULAR 3    /* held rows dependent or reduced Hessian not positive definite: J is NaN                     */
 int tmpc_feedback_jacobian(tmpc_handle* h, double* J, int32_t* jstatus, int dst_is_host, void* cuda_stream);
 
+/* Vector-Jacobian product of the solution map (reverse mode of tmpc_feedback_jacobian), for B solutions:
+ *     G_x0[b*nx + j] = sum_i V_u0[b*nu + i] du0_i/dx0_j + sum_e V_w[b*n_w + e] dw_e/dx0_j,
+ * with the held set, the derivative and the jstatus values (TMPC_JAC_*) of tmpc_feedback_jacobian; G_x0 is NaN for statuses 2
+ * and 3.  K = [H J_A'; J_A 0] is symmetric, so v' dw/dx0 is the init-row block mu of K [y; mu] = [v; 0]: ONE QP solve per
+ * instance for both cotangents together, against nx for the Jacobian.
+ * The solution: W (B*n_w), LAM (B*n_g), status (B) as a step returned them (W_dev, LAM_dev, status_dev of tmpc_step) and
+ * `phase` = the phase that step used (its index mod p before the step, in [0, p)).  They are copied and linearised again in
+ * buffers of the VJP, so a solution stored before later steps gives the same result as right after its step.  W == NULL selects
+ * the last step's own solutions, status, phase and linearisation records; LAM and status must then be NULL and B equal that
+ * step's batch size.  V_u0 (B*nu) and V_w (B*n_w) are the cotangents; either may be NULL, not both.
+ * Buffers: all host memory if is_host != 0, else device memory on the handle's device (runs on `cuda_stream`).  Returns after its
+ * kernels have finished.  Leaves the warm start, the phase index, the linearisation records, the QP step and multipliers, the
+ * log, counters and timing unchanged.
+ * API errors: the handle uses the Gauss-Newton Hessian (hessian_exact = 0 and not economic); a step is in flight; W == NULL and
+ * no step has finished since tmpc_create / tmpc_reset; phase outside [0, p); both cotangents NULL.  B = 0 returns 0. */
+int tmpc_solution_vjp(tmpc_handle* h, int64_t B, const double* W, const double* LAM, const int32_t* status, int32_t phase,
+                      const double* V_u0, const double* V_w, double* G_x0, int32_t* jstatus, int is_host, void* cuda_stream);
+
 /* plant = model integrator: Xn_dev[b] = F(X_dev[b], U_dev[b])   (closed_loop_tools.py:102) */
 int tmpc_plant_step(tmpc_handle* h, const double* X_dev, const double* U_dev, int64_t B, double* Xn_dev,
                     void* cuda_stream);
+
+/* plant Jacobian: JF_dev[b] = [dF/dx | dF/du] at (X_dev[b], U_dev[b]), nx x (nx+nu) row-major per instance, the first-order
+ * sensitivities of the integrator of tmpc_plant_step (those of tmpc_stage_eval_host with order 1) */
+int tmpc_plant_jacobian(tmpc_handle* h, const double* X_dev, const double* U_dev, int64_t B, double* JF_dev, void* cuda_stream);
 
 /* closed-loop log of one (x,u) sample per instance: l_dev[b] = l(x_b,u_b) (economic stage cost of the model card),
  * h_dev[b*nh+i] = (C z_b + c)_i; either may be NULL   (closed_loop_tools.py:64-65, 98-99) */

@@ -34,11 +34,14 @@
 #define NU TMPC_NUM
 #include "tmpc_lin2.cuh"
 
-// thread-per-instance QP kernel (tmpc_qp_thread.cu) and feedback Jacobian (tmpc_fbjac_thread.cu)
+// thread-per-instance QP kernel (tmpc_qp_thread.cu), feedback Jacobian (tmpc_fbjac_thread.cu) and solution VJP (tmpc_vjp_thread.cu)
 cudaError_t tm_launch_qp_thread(const TmProb& P, const TmState& S, const int* list, int cnt, const int* cnt_dev,
                                 double* wsbase, size_t ws_per_inst, int nblocks, int* work_counter, cudaStream_t st);
 cudaError_t tm_launch_fbjac_thread(const TmProb& P, const TmState& S, int cnt, double* wsbase, size_t ws_per_inst, int nblocks,
                                    int* work_counter, double* J, int* jst, cudaStream_t st);
+cudaError_t tm_launch_vjp_thread(const TmProb& P, const TmState& S, int cnt, double* wsbase, size_t ws_per_inst, int nblocks,
+                                 int* work_counter, const double* Vu0, const double* Vw, double* dscr, double* lscr, double* G,
+                                 int* jst, cudaStream_t st);
 int tm_qp_thread_block();
 
 #define QP_WARPS 2          /* warps (instances) per CTA in the warp-per-instance kernels */
@@ -99,6 +102,14 @@ struct tmpc_handle {
   double* jac_buf = nullptr;        // device staging of J and jstatus for host destinations
   int* jst_buf = nullptr;
   int64_t jac_cap = 0;
+  // ---- solution VJP (tmpc_solution_vjp): a stored solution, its linearisation records and the solve's scratch, grown with B
+  bool vjp_smem = false;            // k_vjp's dynamic shared-memory limit raised
+  int64_t vjp_cap = 0;
+  double *vjp_W = nullptr, *vjp_L = nullptr, *vjp_LIN = nullptr, *vjp_D = nullptr, *vjp_LQ = nullptr;
+  int* vjp_st = nullptr;
+  int64_t vjp_io_cap = 0;           // device staging of the cotangents and results for host buffers
+  double *vjp_Vu = nullptr, *vjp_Vw = nullptr, *vjp_G = nullptr;
+  int* vjp_js = nullptr;
 };
 
 static int fail(tmpc_handle* h, const char* what, cudaError_t e) {
@@ -202,6 +213,21 @@ __global__ void __launch_bounds__(QP_WARPS * 32) k_fbjac(TmProb P, TmState S, in
   tm_qpws_carve(smem + (size_t)wid * per, P.N, P.nh, P.nxt, P.maxact, ws, cold + ((size_t)blockIdx.x * W + wid) * cper);
   for (int64_t inst = (int64_t)blockIdx.x * W + wid; inst < cnt; inst += (int64_t)gridDim.x * W) {
     tm_feedback_jacobian(P, S, inst, ws, J, jst);
+    __syncwarp();
+  }
+}
+
+// solution VJP (tm_solution_vjp): warp per instance on the k_qp workspace
+__global__ void __launch_bounds__(QP_WARPS * 32) k_vjp(TmProb P, TmState S, int cnt, double* cold, const double* Vu0,
+                                                     const double* Vw, double* dscr, double* lscr, double* G, int* jst) {
+  extern __shared__ double smem[];
+  const int wid = threadIdx.x / 32, W = blockDim.x / 32;
+  const size_t cper = tm_qpws_cold_doubles(P.N, P.nh, P.nxt, P.maxact);
+  const size_t per = tm_qpws_doubles(P.N, P.nh, P.nxt, P.maxact) - cper;
+  TmQpWs ws;
+  tm_qpws_carve(smem + (size_t)wid * per, P.N, P.nh, P.nxt, P.maxact, ws, cold + ((size_t)blockIdx.x * W + wid) * cper);
+  for (int64_t inst = (int64_t)blockIdx.x * W + wid; inst < cnt; inst += (int64_t)gridDim.x * W) {
+    tm_solution_vjp(P, S, inst, ws, Vu0, Vw, dscr, lscr, G, jst);
     __syncwarp();
   }
 }
@@ -336,6 +362,31 @@ __global__ void k_plant(const double* X, const double* U, int64_t B, double* Xn)
   for (int a = 0; a < NX; ++a) Xn[b * NX + a] = xf[a];
 }
 
+// plant Jacobian JF[b] = [dF/dx | dF/du] (nx x (nx+nu), row-major) at (X[b], U[b]): first-order sensitivities of the same
+// integrator as k_plant, one direction per tm_integrate<1> call (RK4, discrete) or one tm_colloc_stage for all directions
+__global__ void k_plant_jac(const double* X, const double* U, int64_t B, double* JF) {
+  const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  double x[NX], u[NUM];
+#pragma unroll
+  for (int a = 0; a < NX; ++a) x[a] = X[b * NX + a];
+#pragma unroll
+  for (int a = 0; a < NUM; ++a) u[a] = U[b * NUM + a];
+  double* J = JF + b * (int64_t)(NX * NZM);
+#if TMPC_COLLOCATION
+  double rec[NX + NX * NZM];
+  tm_colloc_stage(x, u, 1, nullptr, rec);
+  for (int e = 0; e < NX * NZM; ++e) J[e] = rec[NX + e];
+#else
+  for (int i = 0; i < NZM; ++i) {
+    double xf[NX], si[NX], sj[NX], t[NX];
+    tm_integrate<1>(x, u, i, i, xf, si, sj, t);
+#pragma unroll
+    for (int a = 0; a < NX; ++a) J[a * NZM + i] = si[a];
+  }
+#endif
+}
+
 // closed-loop log of one (x,u) sample per instance: economic stage cost l(x,u) and the path constraint values h = C z + c
 // (tunempc/closed_loop_tools.py:64-65, 98-99)
 __global__ void k_stage_log(const double* X, const double* U, int64_t B, const double* C, const double* c, int nh,
@@ -396,10 +447,9 @@ __global__ void k_sort_scatter(const int* list, int cnt, const int* key, int* bi
   out[atomicAdd(&bins[SORT_BINS + k], 1)] = inst;
 }
 
-// linearise `cnt` instances (list == nullptr: identity) at the iterate (trial = 0) or at the trial point (trial = 1)
-static cudaError_t launch_lin(tmpc_handle* h, const int* list, int64_t cnt, int trial, cudaStream_t st) {
+// linearise `cnt` instances of S (list == nullptr: identity) at the iterate (trial = 0) or at the trial point (trial = 1)
+static cudaError_t launch_lin(tmpc_handle* h, const TmState& S, const int* list, int64_t cnt, int trial, cudaStream_t st) {
   const TmProb& P = h->P;
-  const TmState& S = h->S;
 #if TMPC_RK4
   if (h->lin_mode == 3) {
     const unsigned grid = (unsigned)((cnt * P.N + LIN3_THREADS - 1) / LIN3_THREADS);
@@ -643,6 +693,9 @@ void tmpc_destroy(tmpc_handle* h) {
   if (h->P.prof_counters) cudaFree(h->P.prof_counters);
   if (h->jac_buf) cudaFree(h->jac_buf);
   if (h->jst_buf) cudaFree(h->jst_buf);
+  for (void* q : {(void*)h->vjp_W, (void*)h->vjp_L, (void*)h->vjp_LIN, (void*)h->vjp_D, (void*)h->vjp_LQ, (void*)h->vjp_st,
+                  (void*)h->vjp_Vu, (void*)h->vjp_Vw, (void*)h->vjp_G, (void*)h->vjp_js})
+    if (q) cudaFree(q);
   if (h->ev_ok) for (int i = 0; i < 8; ++i) cudaEventDestroy(h->ev[i]);
   delete h;
 }
@@ -800,12 +853,12 @@ int tmpc_step(tmpc_handle* h, const double* X0_dev, int64_t B, double* U0_dev, d
   const bool was_uniform = h->uniform_ws;   // first step after reset: no per-instance QP cost history yet
   if (h->uniform_ws && B > 1) {
     // right after reset every instance starts from the same (w0, lam0): linearise one and replicate the record
-    CK(launch_lin(h, nullptr, 1, 0, st));
+    CK(launch_lin(h, S, nullptr, 1, 0, st));
     const int64_t nrec = (int64_t)P.N * TM_LSZ;
     k_bcast<<<(unsigned)(((B - 1) * nrec + 255) / 256), 256, 0, st>>>(S.LIN + nrec, S.LIN, B - 1, (int)nrec);
     ++launches; n_lin -= (B - 1) * P.N;
   } else {
-    CK(launch_lin(h, nullptr, B, 0, st));
+    CK(launch_lin(h, S, nullptr, B, 0, st));
   }
   h->uniform_ws = false;
   CK(cudaEventRecord(h->ev[1], st));
@@ -865,7 +918,7 @@ int tmpc_step(tmpc_handle* h, const double* X0_dev, int64_t B, double* U0_dev, d
       if (pass == 0 && !q0) break;
     }
     CK(cudaEventRecord(h->ev[1], st));
-    CK(launch_lin(h, cur, nact, 1, st));
+    CK(launch_lin(h, S, cur, nact, 1, st));
     CK(cudaEventRecord(h->ev[2], st));
     k_post<<<wb, QP_WARPS * 32, 0, st>>>(P, S, cur, (int)nact);
     CK(cudaEventRecord(h->ev[3], st));
@@ -883,7 +936,7 @@ int tmpc_step(tmpc_handle* h, const double* X0_dev, int64_t B, double* U0_dev, d
     }
     if (hc[1] > 0) {   // damped steps: re-linearise at the accepted point, then test convergence
       CK(cudaEventRecord(h->ev[0], st));
-      CK(launch_lin(h, S.list_relin, hc[1], 0, st));
+      CK(launch_lin(h, S, S.list_relin, hc[1], 0, st));
       CK(cudaEventRecord(h->ev[1], st));
       k_conv<<<(unsigned)((hc[1] + QP_WARPS - 1) / QP_WARPS), QP_WARPS * 32, 0, st>>>(P, S, S.list_relin, S.cnt_relin);
       CK(cudaEventRecord(h->ev[2], st));
@@ -1090,6 +1143,127 @@ int tmpc_feedback_jacobian(tmpc_handle* h, double* J, int32_t* jstatus, int dst_
     CK(cudaMemcpyAsync(jstatus, jsd, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost, st));
   }
   CK(cudaStreamSynchronize(st));
+  return 0;
+}
+
+static int vjp_capacity(tmpc_handle* h, int64_t B, bool io) {
+  const TmProb& P = h->P;
+  const size_t b = (size_t)B;
+  if (h->vjp_cap < B) {
+    for (void** q : {(void**)&h->vjp_W, (void**)&h->vjp_L, (void**)&h->vjp_LIN, (void**)&h->vjp_D, (void**)&h->vjp_LQ,
+                     (void**)&h->vjp_st}) {
+      if (*q) cudaFree(*q);
+      *q = nullptr;
+    }
+    h->vjp_cap = 0;
+    CK(cudaMalloc(&h->vjp_W, b * P.n_w * sizeof(double)));
+    CK(cudaMalloc(&h->vjp_L, b * P.n_g * sizeof(double)));
+    CK(cudaMalloc(&h->vjp_LIN, b * P.N * TM_LSZ * sizeof(double)));
+    CK(cudaMalloc(&h->vjp_D, b * P.n_w * sizeof(double)));
+    CK(cudaMalloc(&h->vjp_LQ, b * P.n_g * sizeof(double)));
+    CK(cudaMalloc(&h->vjp_st, b * sizeof(int)));
+    h->vjp_cap = B;
+  }
+  if (io && h->vjp_io_cap < B) {
+    for (void** q : {(void**)&h->vjp_Vu, (void**)&h->vjp_Vw, (void**)&h->vjp_G, (void**)&h->vjp_js}) {
+      if (*q) cudaFree(*q);
+      *q = nullptr;
+    }
+    h->vjp_io_cap = 0;
+    CK(cudaMalloc(&h->vjp_Vu, b * NUM * sizeof(double)));
+    CK(cudaMalloc(&h->vjp_Vw, b * P.n_w * sizeof(double)));
+    CK(cudaMalloc(&h->vjp_G, b * NX * sizeof(double)));
+    CK(cudaMalloc(&h->vjp_js, b * sizeof(int)));
+    h->vjp_io_cap = B;
+  }
+  return 0;
+}
+
+int tmpc_solution_vjp(tmpc_handle* h, int64_t B, const double* W, const double* LAM, const int32_t* status, int32_t phase,
+                      const double* V_u0, const double* V_w, double* G_x0, int32_t* jstatus, int is_host, void* cuda_stream) {
+  if (!h) return 1;
+  if (step_in_flight(h)) { h->err = "tmpc_solution_vjp: a step started by tmpc_step_async is still in flight (call tmpc_wait first)"; return 1; }
+  if (!h->P.hessian_exact) { h->err = "tmpc_solution_vjp: needs the exact Hessian (a Gauss-Newton controller's linearisation has no second-order term)"; return 1; }
+  if (B < 0) { h->err = "tmpc_solution_vjp: negative batch size"; return 1; }
+  const TmProb& P = h->P;
+  const bool stored = W == nullptr;
+  if (stored) {
+    if (LAM || status) { h->err = "tmpc_solution_vjp: W == NULL selects the last step's solutions: LAM and status must be NULL too"; return 1; }
+    if (!h->solved) { h->err = "tmpc_solution_vjp: W == NULL and no step has finished since tmpc_create / tmpc_reset"; return 1; }
+    if (B != h->S.B) { h->err = "tmpc_solution_vjp: W == NULL needs B equal to the last step's batch size"; return 1; }
+  } else {
+    if (!LAM || !status) { h->err = "tmpc_solution_vjp: W, LAM and status are given together"; return 1; }
+    if (phase < 0 || phase >= P.p) { h->err = "tmpc_solution_vjp: phase outside [0, p)"; return 1; }
+  }
+  if (!V_u0 && !V_w) { h->err = "tmpc_solution_vjp: both cotangents are NULL"; return 1; }
+  if (B == 0) return 0;
+  if (!G_x0 || !jstatus) { h->err = "tmpc_solution_vjp: G_x0 and jstatus are required"; return 1; }
+  cudaSetDevice(h->device);
+  cudaStream_t st = (cudaStream_t)cuda_stream;
+  if (vjp_capacity(h, B, is_host != 0)) return 1;
+  const size_t b = (size_t)B;
+  const cudaMemcpyKind kin = is_host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
+  const double* Vu = V_u0;
+  const double* Vw = V_w;
+  double* Gd = G_x0;
+  int* jsd = (int*)jstatus;
+  if (is_host) {
+    if (V_u0) CK(cudaMemcpyAsync(h->vjp_Vu, V_u0, b * NUM * sizeof(double), kin, st));
+    if (V_w) CK(cudaMemcpyAsync(h->vjp_Vw, V_w, b * P.n_w * sizeof(double), kin, st));
+    Vu = V_u0 ? h->vjp_Vu : nullptr;
+    Vw = V_w ? h->vjp_Vw : nullptr;
+    Gd = h->vjp_G;
+    jsd = h->vjp_js;
+  }
+  // The solution, its status and its linearisation records.  W == NULL: the last step's, read in place (after its warm-start
+  // shift the solutions live in Wsh / Lsh and LIN holds the linearisation at them, as for tmpc_feedback_jacobian).  Otherwise a
+  // copy in the VJP's own buffers, linearised again there with the step's dispatch: the handle's W, LAM, LIN, D and LAMQ stay
+  // untouched.  X0 only has to be readable (the solve replaces the x_0 offset that tm_qp_setup forms from it).
+  TmState Sv = h->S;
+  Sv.B = B;
+  if (stored) {
+    Sv.W = h->Wsh;
+    Sv.LAM = h->Lsh;
+  } else {
+    CK(cudaMemcpyAsync(h->vjp_W, W, b * P.n_w * sizeof(double), kin, st));
+    CK(cudaMemcpyAsync(h->vjp_L, LAM, b * P.n_g * sizeof(double), kin, st));
+    CK(cudaMemcpyAsync(h->vjp_st, status, b * sizeof(int), kin, st));
+    Sv.W = h->vjp_W;
+    Sv.LAM = h->vjp_L;
+    Sv.LIN = h->vjp_LIN;
+    Sv.status = h->vjp_st;
+    Sv.phase = phase;
+    CK(launch_lin(h, Sv, nullptr, B, 0, st));
+  }
+  Sv.X0 = Sv.W;
+  const bool use_thread = h->qp_mode == 1 || (h->qp_mode == 2 && B >= h->qp_thread_min);
+  if (use_thread) {
+    CK(tm_launch_vjp_thread(P, Sv, (int)B, h->qp_ws, h->qp_ws_per_inst, h->qp_blocks, h->qp_counter, Vu, Vw, h->vjp_D, h->vjp_LQ,
+                            Gd, jsd, st));
+  } else {
+    if (!h->vjp_smem) {
+      CK(cudaFuncSetAttribute(k_vjp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->qp_smem));
+      h->vjp_smem = true;
+    }
+    k_vjp<<<(unsigned)std::min<int64_t>((B + h->qp_warps - 1) / h->qp_warps, h->qp_wgrid), h->qp_warps * 32, h->qp_smem, st>>>(
+        P, Sv, (int)B, h->qp_cold, Vu, Vw, h->vjp_D, h->vjp_LQ, Gd, jsd);
+    CK(cudaGetLastError());
+  }
+  if (is_host) {
+    CK(cudaMemcpyAsync(G_x0, Gd, b * NX * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(jstatus, jsd, b * sizeof(int), cudaMemcpyDeviceToHost, st));
+  }
+  CK(cudaStreamSynchronize(st));
+  return 0;
+}
+
+int tmpc_plant_jacobian(tmpc_handle* h, const double* X_dev, const double* U_dev, int64_t B, double* JF_dev, void* cuda_stream) {
+  if (!h) return 1;
+  if (B < 0) { h->err = "tmpc_plant_jacobian: negative batch size"; return 1; }
+  if (B == 0) return 0;
+  cudaSetDevice(h->device);
+  k_plant_jac<<<(unsigned)((B + 127) / 128), 128, 0, (cudaStream_t)cuda_stream>>>(X_dev, U_dev, B, JF_dev);
+  CK(cudaGetLastError());
   return 0;
 }
 

@@ -1375,56 +1375,65 @@ TM_HD void tm_pd_check(const TmProb& P, const TmState& S, int64_t inst, TmQpWs& 
   TM_SYNC();
 }
 
-// Feedback Jacobian du0*/dx0 of a converged instance (tmpc_feedback_jacobian, include/tmpc.h).  Held set A = the equality rows +
-// the inequality rows with a non-zero multiplier (stage-0 rows of relax0 excluded), as in tm_pd_check.  Column j is the u_0 block
-// of the linear response of the base QP at the solution (exact Hessian, rows of A held, every offset zero) to the x_0 offset e_j:
-// the KKT system [H J_A'; J_A 0] [dw; dlam] = [0; e_j on the init rows], i.e. the implicit-function derivative of the solution
-// map under strict complementarity.  Same perturbed solve as the tabulation of the first QP (tm_qp0_build_row).  LIN must be
-// valid at (W, LAM); S.D / S.LAMQ of the instance are used as scratch.  J: B*NUM*NX, row-major (nu, nx) per instance; jst: B.
 #define TMPC_JAC_OK 0                   /* the jstatus values of include/tmpc.h (the CPU twin compiles this file without it) */
 #define TMPC_JAC_WEAK 1
 #define TMPC_JAC_NOT_SOLVED 2
 #define TMPC_JAC_SINGULAR 3
-TM_HD void tm_feedback_jacobian(const TmProb& P, const TmState& S, int64_t inst, TmQpWs& ws, double* J, int* jst) {
+
+// The prelude of the sensitivities of a converged instance (tm_feedback_jacobian, tm_solution_vjp).  Held set A = the equality
+// rows + the inequality rows with a non-zero multiplier (stage-0 rows of relax0 excluded), as in tm_pd_check.  Returns
+// TMPC_JAC_NOT_SOLVED when the step's status is not 0 (nothing set up); else TMPC_JAC_OK or TMPC_JAC_WEAK (strict complementarity
+// fails), with A in `mask` and ws the base QP at (W, LAM) with the exact Hessian, the residuals of the held and of the nonlinear
+// rows zeroed: they are O(tol) at a solution and would enter every perturbed solve.  LIN must be valid at (W, LAM).
+TM_HD int tm_jac_prelude(const TmProb& P, const TmState& S, int64_t inst, TmQpWs& ws, unsigned* mask) {
   const int lane = TM_LANE;
   const int NI = P.N * P.nh;
-  double* Ji = J + inst * (int64_t)(NUM * NX);
-  int res = TMPC_JAC_NOT_SOLVED;
-  if (S.status[inst] == 0) {
-    unsigned mask[TM_ALW];
-    for (int wd = 0; wd < TM_ALW; ++wd) mask[wd] = 0u;
-    const double* lam = S.LAM + inst * P.n_g;
-    for (int e = 0; e < NI; ++e) {
-      const int k = e / P.nh, i = e % P.nh;
-      if (k == 0 && P.relax0[i]) continue;
-      if (lam[tm_gh(P, k) + i] != 0.0) tm_mask_set(mask, e);
-    }
-    tm_pin_soft_slacks(P, mask);
-    tm_qp_setup(P, S, inst, ws, 1);
-    // strict complementarity: every held row with a multiplier above lam_tresh, every other row strictly inactive
-    int weak = 0;
-    for (int e = lane; e < NI; e += TM_NL) {
-      const int k = e / P.nh, i = e % P.nh;
-      if (k == 0 && P.relax0[i]) continue;
-      if (tm_mask_get(mask, e)) weak |= fabs(lam[tm_gh(P, k) + i]) < P.lam_tresh;
-      else weak |= ws.hv[e] < 10.0 * P.tol;
-    }
-    weak = tm_wany(weak);
-    // the perturbed solve zeroes the gradient, the dynamics defects and the terminal residuals; the residuals of the held rows
-    // and of the nonlinear rows are O(tol) at a solution and would enter every column
-    TM_SYNC();
-    for (int e = lane; e < NI; e += TM_NL) ws.hv[e] = 0.0;
+  if (S.status[inst] != 0) return TMPC_JAC_NOT_SOLVED;
+  for (int wd = 0; wd < TM_ALW; ++wd) mask[wd] = 0u;
+  const double* lam = S.LAM + inst * P.n_g;
+  for (int e = 0; e < NI; ++e) {
+    const int k = e / P.nh, i = e % P.nh;
+    if (k == 0 && P.relax0[i]) continue;
+    if (lam[tm_gh(P, k) + i] != 0.0) tm_mask_set(mask, e);
+  }
+  tm_pin_soft_slacks(P, mask);
+  tm_qp_setup(P, S, inst, ws, 1);
+  // strict complementarity: every held row with a multiplier above lam_tresh, every other row strictly inactive
+  int weak = 0;
+  for (int e = lane; e < NI; e += TM_NL) {
+    const int k = e / P.nh, i = e % P.nh;
+    if (k == 0 && P.relax0[i]) continue;
+    if (tm_mask_get(mask, e)) weak |= fabs(lam[tm_gh(P, k) + i]) < P.lam_tresh;
+    else weak |= ws.hv[e] < 10.0 * P.tol;
+  }
+  weak = tm_wany(weak);
+  TM_SYNC();
+  for (int e = lane; e < NI; e += TM_NL) ws.hv[e] = 0.0;
 #if NS > 0
-    for (int e = lane; e < P.N * NS; e += TM_NL) ws.gv[e] = 0.0;
+  for (int e = lane; e < P.N * NS; e += TM_NL) ws.gv[e] = 0.0;
 #endif
-    TM_SYNC();
+  TM_SYNC();
+  return weak ? TMPC_JAC_WEAK : TMPC_JAC_OK;
+}
+
+// Feedback Jacobian du0*/dx0 of a converged instance (tmpc_feedback_jacobian, include/tmpc.h).  Column j is the u_0 block of the
+// linear response of the base QP at the solution (exact Hessian, rows of A held, every offset zero) to the x_0 offset e_j: the
+// KKT system [H J_A'; J_A 0] [dw; dlam] = [0; e_j on the init rows], i.e. the implicit-function derivative of the solution map
+// under strict complementarity.  Same perturbed solve as the tabulation of the first QP (tm_qp0_build_row).  LIN must be valid at
+// (W, LAM); S.D / S.LAMQ of the instance are used as scratch.  J: B*NUM*NX, row-major (nu, nx) per instance; jst: B.
+TM_HD void tm_feedback_jacobian(const TmProb& P, const TmState& S, int64_t inst, TmQpWs& ws, double* J, int* jst) {
+  const int lane = TM_LANE;
+  double* Ji = J + inst * (int64_t)(NUM * NX);
+  unsigned mask[TM_ALW];
+  int res = tm_jac_prelude(P, S, inst, ws, mask);
+  if (res != TMPC_JAC_NOT_SOLVED) {
+    // the perturbed solve zeroes the gradient, the dynamics defects and the terminal residuals
     TmQpPert pt;
     pt.homog = 1;
     pt.row = -1;
     pt.dout = S.D + inst * P.n_w;
     pt.lout = S.LAMQ + inst * P.n_g;
     unsigned nxtm[TM_ALW];
-    res = weak ? TMPC_JAC_WEAK : TMPC_JAC_OK;
     for (int j = 0; j < NX; ++j) {
       pt.e0_unit = j;
       int nwrong = 0, ngi = 0;
@@ -1434,6 +1443,57 @@ TM_HD void tm_feedback_jacobian(const TmProb& P, const TmState& S, int64_t inst,
   }
   if (res >= TMPC_JAC_NOT_SOLVED)
     for (int e = lane; e < NUM * NX; e += TM_NL) Ji[e] = NAN;
+  if (lane == 0) jst[inst] = res;
+  TM_SYNC();
+}
+
+// Vector-Jacobian product of the solution map of a converged instance (tmpc_solution_vjp, include/tmpc.h): for the cotangents
+// v_u0 on u_0 and v_w on w, G = v_u0' du0/dx0 + v_w' dw/dx0, with the held set, weak test and statuses of tm_feedback_jacobian.
+// K = [H J_A'; J_A 0] is symmetric, so with v = v_w + v_u0 on the u_0 block, v' dw/dx0 = [v; 0]' K^-1 [0; E] is the init-row
+// block of the solution of K [y; mu] = [v; 0]: the base QP at the solution with the gradient -v and every other offset zero
+// (x_0 offset, dynamics defects, terminal residuals, held-row residuals), one solve whatever nx; G = mu (its sign checked against
+// v' J with tm_feedback_jacobian's J).  Vu0: B*NUM or nullptr,
+// Vw: B*n_w or nullptr; dscr / lscr: B*n_w / B*n_g scratch for the step and multipliers of the solve; G: B*NX; jst: B.
+TM_HD void tm_solution_vjp(const TmProb& P, const TmState& S, int64_t inst, TmQpWs& ws, const double* Vu0, const double* Vw,
+                           double* dscr, double* lscr, double* G, int* jst) {
+  const int lane = TM_LANE;
+  double* Gi = G + inst * NX;
+  unsigned mask[TM_ALW];
+  int res = tm_jac_prelude(P, S, inst, ws, mask);
+  if (res != TMPC_JAC_NOT_SOLVED) {
+    const double* vw = Vw ? Vw + inst * P.n_w : nullptr;
+    const double* vu = Vu0 ? Vu0 + inst * NUM : nullptr;
+    // The QP's stage recursion has no gradient on x_N (the NLP has no terminal cost): the cotangent on x_N enters through the
+    // held last dynamics row, d_N = [A B]_{N-1} d_{N-1}, as [A B]_{N-1}' v_N on stage N-1.  The objective is unchanged on the
+    // feasible set, so is the optimal value and with it the init-row multipliers.
+    for (int e = lane; e < (P.N + 1) * NZ; e += TM_NL) {
+      double v = 0.0;
+      if (e < P.N * NZ) {
+        if (vw) v = vw[e];
+        if (vu && e >= NX && e < NX + NUM) v += vu[e - NX];
+        if (vw && e >= (P.N - 1) * NZ) {
+          const int c = e - (P.N - 1) * NZ;
+          for (int a = 0; a < NX; ++a) v += ws.AB[(size_t)(P.N - 1) * NX * NZ + a * NZ + c] * vw[P.N * NZ + a];
+        }
+      }
+      ws.r[e] = -v;
+    }
+    for (int e = lane; e < P.N * NX; e += TM_NL) ws.b[e] = 0.0;
+    for (int t = lane; t < P.nxt; t += TM_NL) ws.tr[t] = 0.0;
+    TM_SYNC();
+    TmQpPert pt;
+    pt.homog = 0;                                            // keep the gradient -v; the x_0 offset is zeroed by the solve
+    pt.e0_unit = -1;
+    pt.row = -1;
+    pt.dout = dscr + inst * P.n_w;
+    pt.lout = lscr + inst * P.n_g;
+    unsigned nxtm[TM_ALW];
+    int nwrong = 0, ngi = 0;
+    if (tm_qp_solve(P, S, inst, ws, mask, nxtm, nwrong, ngi, &pt) != 0) res = TMPC_JAC_SINGULAR;
+    else for (int j = lane; j < NX; j += TM_NL) Gi[j] = pt.lout[j];
+  }
+  if (res >= TMPC_JAC_NOT_SOLVED)
+    for (int j = lane; j < NX; j += TM_NL) Gi[j] = NAN;
   if (lane == 0) jst[inst] = res;
   TM_SYNC();
 }

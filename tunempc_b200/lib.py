@@ -18,10 +18,10 @@ _dp = ctypes.POINTER(ctypes.c_double)
 _ip = ctypes.POINTER(ctypes.c_int32)
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-shared", "-Xcompiler", "-fPIC",
-              "-std=c++17", "--threads", "3"]      # the three translation units of a model library compile side by side
+              "-std=c++17", "--threads", "4"]      # the four translation units of a model library compile side by side
 
 EXPORTS = ["tmpc_default_opts", "tmpc_model_info", "tmpc_model_slacks", "tmpc_create", "tmpc_destroy", "tmpc_last_error",
-           "tmpc_set_tables", "tmpc_reset", "tmpc_get_index", "tmpc_step", "tmpc_step_async", "tmpc_wait", "tmpc_busy", "tmpc_step_host", "tmpc_feedback_jacobian", "tmpc_plant_step", "tmpc_stage_log",
+           "tmpc_set_tables", "tmpc_reset", "tmpc_get_index", "tmpc_step", "tmpc_step_async", "tmpc_wait", "tmpc_busy", "tmpc_step_host", "tmpc_feedback_jacobian", "tmpc_solution_vjp", "tmpc_plant_step", "tmpc_plant_jacobian", "tmpc_stage_log",
            "tmpc_get_log", "tmpc_get_counters", "tmpc_get_timing", "tmpc_stage_eval_host", "tmpc_fp64_peak"]
 
 
@@ -45,14 +45,15 @@ def build_model_lib(name, force=False, verbose=False):
     """nvcc-compile libtmpc_<name>.so in-tree for sm_100a (cross-compiles without a GPU)."""
     out = lib_path(name)
     srcs = [os.path.join(_PKG, "csrc", "tmpc.cu"), os.path.join(_PKG, "csrc", "tmpc_qp_thread.cu"),
-            os.path.join(_PKG, "csrc", "tmpc_fbjac_thread.cu"), os.path.join(_PKG, "csrc", "tmpc_qp_thread.cuh"),
+            os.path.join(_PKG, "csrc", "tmpc_fbjac_thread.cu"), os.path.join(_PKG, "csrc", "tmpc_vjp_thread.cu"),
+            os.path.join(_PKG, "csrc", "tmpc_qp_thread.cuh"),
             os.path.join(_PKG, "csrc", "tmpc_core.cuh"), os.path.join(_PKG, "csrc", "tmpc_lin2.cuh"),
             os.path.join(_PKG, "csrc", "tmpc_qp.cuh"), os.path.join(_PKG, "csrc", "tmpc_lin3.cuh"),
             os.path.join(_PKG, "csrc", "gen", "model_%s.h" % name), os.path.join(_ROOT, "include", "tmpc.h")]
     if not force and os.path.exists(out) and all(os.path.getmtime(out) >= os.path.getmtime(s) for s in srcs):
         return out
     cmd = ["nvcc"] + NVCC_FLAGS + ['-DTMPC_MODEL_HEADER="gen/model_%s.h"' % name, "-I" + os.path.join(_ROOT, "include"),
-                                  "-I" + os.path.join(_PKG, "csrc"), srcs[0], srcs[1], srcs[2], "-o", out]
+                                  "-I" + os.path.join(_PKG, "csrc"), srcs[0], srcs[1], srcs[2], srcs[3], "-o", out]
     if verbose:
         cmd.insert(1, "-Xptxas=-v")
     subprocess.check_call(cmd)
@@ -87,7 +88,9 @@ class ModelLib:
         L.tmpc_busy.argtypes = [vp, _ip]
         L.tmpc_step_host.argtypes = [vp, vp, ctypes.c_int64, vp, vp, vp, vp, vp, vp, vp]
         L.tmpc_feedback_jacobian.argtypes = [vp, vp, vp, ctypes.c_int, vp]
+        L.tmpc_solution_vjp.argtypes = [vp, ctypes.c_int64, vp, vp, vp, ctypes.c_int32, vp, vp, vp, vp, ctypes.c_int, vp]
         L.tmpc_plant_step.argtypes = [vp, vp, vp, ctypes.c_int64, vp, vp]
+        L.tmpc_plant_jacobian.argtypes = [vp, vp, vp, ctypes.c_int64, vp, vp]
         L.tmpc_stage_log.argtypes = [vp, vp, vp, ctypes.c_int64, vp, vp, vp]
         L.tmpc_get_log.argtypes = [vp, vp, vp, vp, vp, ctypes.c_int]
         L.tmpc_get_counters.argtypes = [vp, ctypes.POINTER(ctypes.c_int64)]

@@ -229,6 +229,7 @@ class Pmpc:
             X0 = x0.contiguous()
             B = X0.shape[0]
             self.__ensure_batch(B)
+            phase = self.__index % pb.p
             dev = X0.device
             full = outputs == "all"
             U0 = torch.empty((B, pb.nu), dtype=torch.float64, device=dev)
@@ -242,7 +243,7 @@ class Pmpc:
             stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
             self.__check(L.tmpc_step(self.__h, ptr(X0), B, ptr(U0), ptr(W), ptr(LAM), ptr(G), ptr(st), ptr(it), ptr(fl),
                                      stream))
-            self.__out = dict(u0=U0, w=W, lam_g=LAM, g=G, status=st, iter=it, flags=fl)
+            self.__out = dict(u0=U0, w=W, lam_g=LAM, g=G, status=st, iter=it, flags=fl, phase=phase)
             self.__log_append(torch_dev=dev)
             self.__index += 1
             return U0
@@ -256,6 +257,7 @@ class Pmpc:
         X0 = np.ascontiguousarray(a)
         B = X0.shape[0]
         self.__ensure_batch(B)
+        phase = self.__index % pb.p
         full = outputs == "all"
         U0 = np.empty((B, pb.nu))
         W = np.empty((B, pb.n_w)) if full else None
@@ -266,7 +268,8 @@ class Pmpc:
         fl = np.empty(B, dtype=np.int32)
         vp = lambda t: ctypes.c_void_p(t.ctypes.data) if t is not None else None
         self.__check(L.tmpc_step_host(self.__h, vp(X0), B, vp(U0), vp(W), vp(LAM), vp(G), vp(st), vp(it), vp(fl)))
-        self.__out = dict(u0=U0, w=W, lam_g=LAM, g=G, status=st, iter=it, flags=fl, single=single_shape is not None)
+        self.__out = dict(u0=U0, w=W, lam_g=LAM, g=G, status=st, iter=it, flags=fl, single=single_shape is not None,
+                          phase=phase)
         self.__log_append()
         self.__index += 1
         if single_shape is not None:
@@ -290,6 +293,7 @@ class Pmpc:
         X0 = X0.contiguous()
         B = X0.shape[0]
         self.__ensure_batch(B)
+        phase = self.__index % pb.p
         dev = X0.device
         full = outputs == "all"
         U0 = torch.empty((B, pb.nu), dtype=torch.float64, device=dev)
@@ -303,7 +307,7 @@ class Pmpc:
         stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
         self.__check(self.__lib.lib.tmpc_step_async(self.__h, ptr(X0), B, ptr(U0), ptr(W), ptr(LAM), ptr(G), ptr(st), ptr(it),
                                                     ptr(fl), stream))
-        self.__pending = dict(out=dict(u0=U0, w=W, lam_g=LAM, g=G, status=st, iter=it, flags=fl), dev=dev, keep=X0)
+        self.__pending = dict(out=dict(u0=U0, w=W, lam_g=LAM, g=G, status=st, iter=it, flags=fl, phase=phase), dev=dev, keep=X0)
         return U0
 
     def busy(self):
@@ -386,6 +390,63 @@ class Pmpc:
             return J[0].copy(), int(js[0])
         return J, js
 
+    def solution_vjp(self, v_u0=None, v_w=None, w=None, lam_g=None, status=None, phase=None):
+        """Vector-Jacobian product of the solution map (C ABI: tmpc_solution_vjp, definition in include/tmpc.h): (G, jstatus) with
+        G (B, nx), G[b] = v_u0[b]' du0/dx0 + v_w[b]' dw/dx0, and jstatus (B,) int32 as in feedback_jacobian() (G is NaN for 2
+        and 3).  One QP solve per instance whatever nx, for both cotangents together.
+        v_u0 (B, nu), v_w (B, n_w): the cotangents; either may be None, not both.
+        w, lam_g, status, phase: a solution as a step returned it (w_sol, lam_g, status, last_phase of that step), which may be
+        several steps old; phase defaults to the last step's.  w=None: the last step's own solutions (lam_g, status and phase must
+        then be None).  torch CUDA tensors for torch inputs (and after a torch step with w=None), numpy arrays otherwise;
+        ((nx,), int) after a single-state step with w=None.  Needs the exact Hessian; changes nothing in the controller."""
+        if getattr(self, "_Pmpc__pending", None) is not None:
+            raise RuntimeError("solution_vjp: a step started by step_async is still in flight (call wait() first)")
+        pb = self.__pb
+        L = self.__lib.lib
+        o = self.__out
+        if w is None:
+            if lam_g is not None or status is not None or phase is not None:
+                raise ValueError("solution_vjp: lam_g, status and phase go with w")
+            B, ph = self.__B, 0
+            is_torch = (o is not None and type(o["u0"]).__module__.startswith("torch")) or any(
+                type(v).__module__.startswith("torch") for v in (v_u0, v_w))
+        else:
+            if lam_g is None or status is None:
+                raise ValueError("solution_vjp: w needs lam_g and status")
+            ph = int(phase) if phase is not None else (o["phase"] if o is not None else 0)
+            is_torch = type(w).__module__.startswith("torch")
+            B = int(w.shape[0])
+        if is_torch:
+            import torch
+            dev = torch.device("cuda", self.__device)
+            f64 = lambda t: None if t is None else torch.as_tensor(t, dtype=torch.float64, device=dev).contiguous()
+            i32 = lambda t: None if t is None else torch.as_tensor(t, dtype=torch.int32, device=dev).contiguous()
+            args = [f64(w), f64(lam_g), i32(status), f64(v_u0), f64(v_w)]
+            G = torch.empty((B, pb.nx), dtype=torch.float64, device=dev)
+            js = torch.empty(B, dtype=torch.int32, device=dev)
+            ptr = lambda t: ctypes.c_void_p(t.data_ptr()) if t is not None else None
+            stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+            is_host = 0
+        else:
+            f64 = lambda t: None if t is None else np.ascontiguousarray(t, dtype=np.float64)
+            i32 = lambda t: None if t is None else np.ascontiguousarray(t, dtype=np.int32)
+            args = [f64(w), f64(lam_g), i32(status), f64(v_u0), f64(v_w)]
+            G = np.empty((B, pb.nx))
+            js = np.empty(B, dtype=np.int32)
+            ptr = lambda t: ctypes.c_void_p(t.ctypes.data) if t is not None else None
+            stream = None
+            is_host = 1
+        for a, n, name in zip(args, (pb.n_w, pb.n_g, 1, pb.nu, pb.n_w), ("w", "lam_g", "status", "v_u0", "v_w")):
+            size = None if a is None else (a.numel() if is_torch else a.size)
+            if size is not None and size != B * n and not (w is None and o is None):   # no step yet: the library reports it
+                raise ValueError("solution_vjp: %s has %d elements, expected %d x %d" % (name, size, B, n))
+        W, LAM, st, Vu, Vw = args
+        self.__check(L.tmpc_solution_vjp(self.__h, B, ptr(W), ptr(LAM), ptr(st), ph, ptr(Vu), ptr(Vw), ptr(G), ptr(js), is_host,
+                                         stream))
+        if w is None and not is_torch and o is not None and o.get("single"):
+            return G[0].copy(), int(js[0])
+        return G, js
+
     # ---- closed loop helpers -------------------------------------------------------------------------
     def plant_step(self, X, U):
         """x+ = F(x,u) for every row (closed_loop_tools.py:102).  torch CUDA tensors in, torch CUDA tensor out."""
@@ -397,6 +458,18 @@ class Pmpc:
         self.__check(self.__lib.lib.tmpc_plant_step(self.__h, ctypes.c_void_p(X.data_ptr()), ctypes.c_void_p(U.data_ptr()),
                                                     X.shape[0], ctypes.c_void_p(Xn.data_ptr()), stream))
         return Xn
+
+    def plant_jacobian(self, X, U):
+        """[dF/dx | dF/du] at every row (C ABI: tmpc_plant_jacobian): torch CUDA tensors in, (B, nx, nx+nu) out."""
+        import torch
+        X = X.contiguous()
+        U = U.contiguous()
+        B = X.shape[0]
+        JF = torch.empty((B, self.__pb.nx, self.__pb.nx + self.__pb.nu), dtype=torch.float64, device=X.device)
+        stream = ctypes.c_void_p(torch.cuda.current_stream(X.device).cuda_stream)
+        self.__check(self.__lib.lib.tmpc_plant_jacobian(self.__h, ctypes.c_void_p(X.data_ptr()), ctypes.c_void_p(U.data_ptr()), B,
+                                                        ctypes.c_void_p(JF.data_ptr()), stream))
+        return JF
 
     def stage_log(self, X, U):
         """l(x,u) and h(x,u) = C z + c for every row (closed_loop_tools.py:64-65, 98-99): torch CUDA tensors in,
@@ -448,6 +521,11 @@ class Pmpc:
     @property
     def status(self):
         return self.__out["status"] if self.__out else None
+
+    @property
+    def last_phase(self):
+        """the phase (index mod p) the last step used: the `phase` that solution_vjp() takes with that step's solution"""
+        return self.__out["phase"] if self.__out else None
 
     @property
     def log(self):
